@@ -242,6 +242,43 @@ def measured_peak_gbs():
     return 6650.0, "fallback (B200_PROFILING.md)"
 
 
+def _gather_sample(bufs, segments, n, rng):
+    """float32 values at n seeded positions of the concatenation of `segments`, each (buffer index, start, length)
+    of a flat device tensor in `bufs`; positions are in ascending order of the concatenation."""
+    import torch
+    seg_buf = np.array([s[0] for s in segments], np.int64)
+    seg_start = np.array([s[1] for s in segments], np.int64)
+    cum = np.concatenate([[0], np.cumsum([s[2] for s in segments], dtype=np.int64)])
+    idx = np.sort(rng.integers(0, cum[-1], n, dtype=np.int64))
+    seg = np.searchsorted(cum, idx, side="right") - 1
+    pos = seg_start[seg] + (idx - cum[seg])
+    parts = []
+    for b, buf in enumerate(bufs):
+        sel = pos[seg_buf[seg] == b]
+        if len(sel):
+            ix = torch.from_numpy(sel).to(buf.device)
+            parts.append(buf.reshape(-1).index_select(0, ix).float().cpu().numpy())
+    return np.concatenate(parts)
+
+
+def dump_outputs(out_dir: Path, pipes, seed: int = 0) -> None:
+    """Write what the last step of the timed path left in the sub-batch buffers, as float32 .npy files (48 MiB in all):
+      pixels.npy        2^23 values of the uint8 RGB output of the whole batch (images in batch order, each (H, W, 3)
+                        row-major, concatenated), at seeded random positions in ascending order
+      coefficients.npy  2^22 values of the int16 quantised coefficients (device order, sub-batches concatenated), the same way
+      errors.npy        every image's device error word
+    The positions depend only on `seed` and the batch, so two builds run with the same arguments compare value for value."""
+    out_dir.mkdir(parents=True, exist_ok=True)
+    rng = np.random.default_rng(seed)
+    outs = [p.out for p in pipes]
+    images = [(c, off, int(np.prod(shape))) for c, p in enumerate(pipes)
+              for off, shape in zip(p.plan.geom.out_offsets, p.plan.geom.out_shapes)]
+    np.save(out_dir / "pixels.npy", _gather_sample(outs, images, 1 << 23, rng))
+    coefs = [p.coef for p in pipes]
+    np.save(out_dir / "coefficients.npy", _gather_sample(coefs, [(c, 0, t.numel()) for c, t in enumerate(coefs)], 1 << 22, rng))
+    np.save(out_dir / "errors.npy", np.concatenate([p.err.cpu().numpy() for p in pipes]).astype(np.float32))
+
+
 def run_reference(args):
     """The reference's algorithm on the host cores: the CPU oracle (C port, oracle/) over all threads."""
     rank = int(os.environ.get("RANK", "0"))
@@ -291,7 +328,13 @@ def main():
     ap.add_argument("--distinct", type=int, default=64, help="distinct synthetic images (cycled to --images)")
     ap.add_argument("--cpu-sample", type=int, default=48, help="images decoded by the 1-core CPU baseline")
     ap.add_argument("--no-configs", action="store_true", help="skip the per-shape `configs` measurements and the Python-reference timing")
+    ap.add_argument("--dump-outputs", type=Path, metavar="DIR",
+                    help="after the timed steps, write a seeded sample of what the last one computed (rank 0) to DIR/*.npy")
     args = ap.parse_args()
+    if args.steps < 1 or args.warmup < 0:
+        ap.error("--steps must be at least 1 and --warmup at least 0")
+    if args.impl == "reference" and args.dump_outputs is not None:
+        ap.error("--dump-outputs applies to --impl b200")
     if args.impl == "reference":
         run_reference(args)
         return
@@ -411,6 +454,8 @@ def main():
     ms_e2e = max_over_ranks(max(ms_ev, ms_wall))
     clocks = sampler.stop()
     assert all(int(e.abs().sum()) == 0 for e in err_hosts), "device reported decode errors"
+    if args.dump_outputs is not None and rank == 0:
+        dump_outputs(args.dump_outputs, pipes)
     launches_per_step = sum(p.kernel_launches_per_step for p in pipes)
     device_bytes = sum(p.device_bytes() for p in pipes)
 
