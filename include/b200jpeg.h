@@ -226,7 +226,7 @@ bj_status bj_entropy_decode(const bj_scan* scans, int scan_first, int n_scans, i
 #define BJ_IN_SAMPLES 1  /* sample buffer produced by BJ_OUT_SAMPLES */
 
 int bj_version(void);
-int bj_sizeof(int what);         /* 0: sizeof(bj_image) -- lets a binding verify its struct mirrors */
+int bj_sizeof(int what);         /* 0: sizeof(bj_image), 1: sizeof(bj_resize_job) -- lets a binding verify its struct mirrors */
 int bj_sizeof_entropy(int what); /* 1: sizeof(bj_scan), 2: sizeof(bj_entropy_buffers), 3: BJ_SUBSEQ_BITS */
 int bj_pixels_fast_strip(int layout); /* MCUs per CTA the specialised pixel kernel uses for BJ_LAYOUT_* (0: generic) */
 const char* bj_last_cuda_error(void);
@@ -309,6 +309,46 @@ void bj_host_read_files(const char* const* paths, const uint64_t* size, const ui
 bj_status bj_pixels(const bj_image* images, int n_images, int max_strips, const void* in, int in_kind,
                     uint64_t total_blocks, const int16_t* qtabs, const double* idct_table_t, void* out, int out_kind,
                     uint32_t layout_mask, uint32_t* stats, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Resize + normalise of decoded images into one (N, 3, h, w) batch tensor (data-loader output).
+ *
+ * Filter: torch.nn.functional.interpolate(mode="bilinear", align_corners=False, antialias=True), separable
+ * triangle filter, weights computed in the kernel (csrc/bj_resize_math.cuh), fp32 accumulation.  Value of an
+ * output element of channel c: v * a[c] + b[c], v the resized value on the 0..255 scale; uint8 output rounds
+ * that to nearest even and clamps to [0, 255].  Greyscale sources give three channels (each with its a/b).
+ * ------------------------------------------------------------------------------------------- */
+#define BJ_DTYPE_U8 0
+#define BJ_DTYPE_F16 1
+#define BJ_DTYPE_BF16 2
+#define BJ_DTYPE_F32 3
+
+/* One source image: 40 bytes, 8-byte aligned. */
+typedef struct bj_resize_job {
+    uint64_t src_offset;   /* byte offset of pixel (0,0) in src (bj_image.out_offset of BJ_OUT_RGB); any alignment */
+    uint32_t src_pitch;    /* bytes per source row (bj_image.out_pitch) */
+    uint32_t channels;     /* 3 (RGB) or 1 (greyscale) */
+    uint32_t x0, y0, x1, y1; /* source box [x0, x1) x [y0, y1) in pixels, x0 < x1 <= width, y0 < y1 <= height */
+    uint32_t dst_index;    /* image slot n of the output tensor */
+    uint32_t reserved;
+} bj_resize_job;
+
+typedef struct bj_resize_params {
+    uint32_t out_h, out_w;  /* output size, 1..65535 */
+    uint32_t dtype;         /* BJ_DTYPE_* */
+    uint32_t channels_last; /* 0: NCHW, 1: NHWC storage of the (N, 3, h, w) tensor */
+    float a[3], b[3];       /* per-channel scale and offset */
+} bj_resize_params;
+
+/*
+ *   jobs   DEVICE array of n_jobs bj_resize_job
+ *   src    decoded uint8 pixels (the BJ_OUT_RGB buffer of bj_pixels)
+ *   dst    output tensor storage, element type dtype, dense NCHW or NHWC
+ *   p      HOST pointer; copied into the kernel parameters (the caller may reuse it when the call returns)
+ * One launch covers every job (grid: output tiles x jobs; more than 65535 jobs are launched in slices).
+ */
+bj_status bj_resize(const bj_resize_job* jobs, int n_jobs, const uint8_t* src, void* dst, const bj_resize_params* p,
+                    void* stream);
 
 #ifdef __cplusplus
 }

@@ -436,7 +436,9 @@ thread_local char g_err[256] = "";
 extern "C" {
 
 int bj_version(void) { return BJ_VERSION; }
-int bj_sizeof(int what) { return what == 0 ? (int)sizeof(bj_image) : -1; }
+int bj_sizeof(int what) {
+    return what == 0 ? (int)sizeof(bj_image) : what == 1 ? (int)sizeof(bj_resize_job) : -1;
+}
 const char* bj_last_cuda_error(void) { return g_err; }
 
 bj_status bj_set_cuda_error(cudaError_t e, const char* where) {
