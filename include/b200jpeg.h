@@ -226,7 +226,8 @@ bj_status bj_entropy_decode(const bj_scan* scans, int scan_first, int n_scans, i
 #define BJ_IN_SAMPLES 1  /* sample buffer produced by BJ_OUT_SAMPLES */
 
 int bj_version(void);
-int bj_sizeof(int what);         /* 0: sizeof(bj_image), 1: sizeof(bj_resize_job) -- lets a binding verify its struct mirrors */
+int bj_sizeof(int what);         /* 0: sizeof(bj_image), 1: sizeof(bj_resize_job), 2: sizeof(bj_scaled_job) -- lets a
+                                    binding verify its struct mirrors */
 int bj_sizeof_entropy(int what); /* 1: sizeof(bj_scan), 2: sizeof(bj_entropy_buffers), 3: BJ_SUBSEQ_BITS */
 int bj_pixels_fast_strip(int layout); /* MCUs per CTA the specialised pixel kernel uses for BJ_LAYOUT_* (0: generic) */
 const char* bj_last_cuda_error(void);
@@ -349,6 +350,37 @@ typedef struct bj_resize_params {
  */
 bj_status bj_resize(const bj_resize_job* jobs, int n_jobs, const uint8_t* src, void* dst, const bj_resize_params* p,
                     void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Reduced-size decode: scale 1/s, s = 2, 4 or 8, in the DCT domain (libjpeg's scale_denom, PIL's draft()).
+ * Output (ceil(H/s), ceil(W/s), 3) or (ceil(H/s), ceil(W/s)); scaled pixel k covers full pixels [k s, (k+1) s), the
+ * encoder's padding included at the right / bottom edge.  Each block of component c gives an NY x NX tile,
+ * NX = 8 (hmax / h_c) / s, NY = 8 (vmax / v_c) / s: the 2-D inverse DCT of the block's low-frequency NX x NY corner
+ * with the cosine argument of an N-point transform (the 8-point IDCT's normalisation, so the block mean is kept),
+ * rounded half to even, + 128; no layout needs chroma upsampling.  Colour: the fp32 rule of the full path, clip,
+ * round half to even.  The arithmetic, with its fp32 error bound, is csrc/bj_scaled_math.cuh.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct bj_scaled_job {   /* 24 bytes */
+    uint64_t out_offset;         /* byte offset of scaled pixel (0,0) in out */
+    uint32_t out_pitch;          /* bytes per row, >= ceil(width/s) * channels */
+    uint32_t image;              /* index into images */
+    uint32_t log2_scale;         /* 1, 2 or 3 */
+    uint32_t reserved;
+} bj_scaled_job;
+
+/*
+ *   images      DEVICE array of bj_image, the records bj_pixels reads; out_offset, out_pitch, strip_mcus and
+ *               strips_per_row are not used
+ *   jobs        DEVICE array of n_jobs bj_scaled_job: any mix of images, layouts and scales
+ *   max_strips  max over jobs of mcus_y * ceil(mcus_x / S), S = min(192 / blocks_per_mcu,
+ *               6144 / (ncomp * 16 * hmax * vmax)) MCUs per CTA
+ *   coef        coefficient buffer (zig-zag, quantised); only the zig-zag prefix each block's corner needs is read
+ *   qtabs       as for bj_pixels
+ *   out         uint8 pixels at each job's out_offset / out_pitch
+ * One launch covers every job (grid: strips x jobs; more than 65535 jobs are launched in slices).
+ */
+bj_status bj_pixels_scaled(const bj_image* images, const bj_scaled_job* jobs, int n_jobs, int max_strips,
+                           const int16_t* coef, const int16_t* qtabs, uint8_t* out, void* stream);
 
 #ifdef __cplusplus
 }

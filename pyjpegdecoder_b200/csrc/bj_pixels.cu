@@ -437,7 +437,8 @@ extern "C" {
 
 int bj_version(void) { return BJ_VERSION; }
 int bj_sizeof(int what) {
-    return what == 0 ? (int)sizeof(bj_image) : what == 1 ? (int)sizeof(bj_resize_job) : -1;
+    return what == 0 ? (int)sizeof(bj_image) : what == 1 ? (int)sizeof(bj_resize_job)
+         : what == 2 ? (int)sizeof(bj_scaled_job) : -1;
 }
 const char* bj_last_cuda_error(void) { return g_err; }
 

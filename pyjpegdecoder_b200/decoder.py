@@ -191,7 +191,7 @@ BATCH_CHUNK = 512
 
 def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Union[str, torch.device]] = None,
                  chunk: Optional[int] = None, on_error: str = "raise", keep_coefficients: bool = False,
-                 to_host: bool = False) -> List[JpegDecoder]:
+                 to_host: bool = False, scale: int = 1, _scales=None) -> List[JpegDecoder]:
     """Decode many files and return one JpegDecoder-like object per file (pixels stay on the device until
     `image_array` is read).  Small batches run as ONE device pipeline (one launch sequence for all files); batches
     larger than 1.5 x `chunk` files are cut into sub-batches of `chunk` files that flow through the streaming front
@@ -208,9 +208,18 @@ def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Unio
 
     to_host=True: the pixels of every sub-batch are also copied to pinned host memory, one transfer per sub-batch
     behind the decode of the next ones; `image_array` (what the reference returns: a numpy array in host memory) is
-    then a view of that copy instead of one pageable device->host copy per image."""
+    then a view of that copy instead of one pageable device->host copy per image.
+
+    scale=2, 4 or 8: every image is decoded at 1/scale of its size in the DCT domain, (ceil(H/s), ceil(W/s), 3), from
+    the low-frequency corner of each block (csrc/bj_scaled_math.cuh); image_tensor, image_array, save() and DLPack give
+    those pixels, image_width / image_height stay the file's.  _scales: per-image scales, or a function
+    (bj_image records of a sub-batch, indices of its files in `files`) -> scales (decode_to_tensor(scale="auto"))."""
+    from .scaled import check_scale
     if on_error not in ("raise", "return"):
         raise ValueError("on_error must be 'raise' or 'return'")
+    scale = check_scale(scale)
+    if _scales is None and scale != 1:
+        _scales = scale
     files = list(files)
     if not files:
         return []
@@ -218,13 +227,14 @@ def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Unio
     if chunk < 1:
         raise ValueError("chunk must be positive")
     if on_error == "return":
-        return _decode_batch_tolerant(files, device, chunk)
+        return _decode_batch_tolerant(files, device, chunk, _scales)
     if len(files) > chunk + chunk // 2:
-        from .loader import decode_stream
+        from .loader import _decode_stream
         out: List[JpegDecoder] = []
-        for part in decode_stream(files, chunk=chunk, device=device, keep_coefficients=keep_coefficients, to_host=to_host):
+        for part in _decode_stream(files, chunk, device, keep_coefficients, to_host, _scales):
             out.extend(part)
         return out
+    scales = _for_files(_scales, np.arange(len(files)))
     from .pipeline import FAST_PLAN_MIN_FILES
     if len(files) >= FAST_PLAN_MIN_FILES and all(isinstance(f, (str, Path)) for f in files):
         # paths: the C helper's threads read the files straight into the pinned staging buffer and walk them
@@ -236,16 +246,24 @@ def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Unio
         except Exception:
             release_pinned(raw)
             raise
-        batch = decode_batch_on_device(None, device=device, packed=(raw, offs), plan=plan)
+        batch = decode_batch_on_device(None, device=device, packed=(raw, offs), plan=plan, scales=scales)
     else:
         datas = [_read(f) for f in files]
-        batch = decode_batch_on_device(datas, device=device)
+        batch = decode_batch_on_device(datas, device=device, scales=scales)
     if to_host:
         batch.start_host_copy()
     return [JpegDecoder(f, _batch=batch, _index=i) for i, f in enumerate(files)]
 
 
-def _decode_batch_tolerant(files: list, device, chunk: int) -> list:
+def _for_files(scales, idx: np.ndarray):
+    """decode_batch_on_device's scales for a sub-batch made of files[idx]: a function of (records, file indices) is
+    bound to the indices."""
+    if callable(scales):
+        return lambda images: scales(images, idx)
+    return scales
+
+
+def _decode_batch_tolerant(files: list, device, chunk: int, scales=None) -> list:
     """decode_batch(on_error="return"): header problems are found per file on the host (the same parser and plan
     checks the batch path runs), entropy-data problems come back as the per-image device error words."""
     from .errors import JpegError
@@ -264,7 +282,8 @@ def _decode_batch_tolerant(files: list, device, chunk: int) -> list:
         good.append(i)
     for a in range(0, len(good), chunk):
         idx = good[a:a + chunk]
-        batch = decode_batch_on_device([datas[i] for i in idx], device=device, check=False)
+        batch = decode_batch_on_device([datas[i] for i in idx], device=device, check=False,
+                                       scales=_for_files(scales, np.asarray(idx)))
         pipe = batch.stats["_pipe"]
         err = pipe.err.cpu().numpy()                          # synchronises
         for k, i in enumerate(idx):

@@ -12,6 +12,7 @@ from concurrent.futures import ThreadPoolExecutor
 from pathlib import Path
 from typing import Iterable, Iterator, List, Optional, Sequence, Union
 
+import numpy as np
 import torch
 
 from .decoder import JpegDecoder, _read
@@ -170,29 +171,38 @@ def _check(batch) -> None:
 
 
 def decode_stream(files: Iterable[Source], chunk: int = 512, device: Optional[Union[str, torch.device]] = None,
-                  keep_coefficients: bool = False, to_host: bool = False) -> Iterator[List[JpegDecoder]]:
+                  keep_coefficients: bool = False, to_host: bool = False, scale: int = 1) -> Iterator[List[JpegDecoder]]:
     """Decode an arbitrarily long sequence of files in sub-batches of at most `chunk` files (the first two are
     smaller, see _chunks); yields one list of JpegDecoder objects per sub-batch, in order.  Errors of a file (NotJpeg, CorruptedJpeg, ...) are raised when its chunk is reached.
     Three things overlap: the worker thread prepares and uploads the chunks ahead, the GPU decodes up to three chunks
     on alternating streams (a chunk is checked only when two later ones have been enqueued), and the caller consumes
-    the oldest finished chunk."""
+    the oldest finished chunk.  scale=2, 4 or 8: reduced-size decode, as in decode_batch."""
+    from .scaled import check_scale
     if chunk < 1:
         raise ValueError("chunk must be positive")
+    scale = check_scale(scale)
+    yield from _decode_stream(files, chunk, device, keep_coefficients, to_host, None if scale == 1 else scale)
+
+
+def _decode_stream(files, chunk, device, keep_coefficients=False, to_host=False, scales=None):
+    """decode_stream with scales: None, one scale, or a function (bj_image records of a sub-batch, indices of its files
+    in `files`) -> per-image scales, called once the sub-batch is planned."""
     up = _Uploader(device)
     it = _chunks(files, chunk)
     depth = _N_SLOTS - 1                     # chunks prepared ahead of the one being enqueued
     try:
-        yield from _stream(up, it, depth, device, keep_coefficients, to_host)
+        yield from _stream(up, it, depth, device, keep_coefficients, to_host, scales)
     finally:
         up.close()
 
 
-def _stream(up, it, depth, device, keep_coefficients=False, to_host=False):
+def _stream(up, it, depth, device, keep_coefficients=False, to_host=False, scales=None):
     # consecutive chunks run on alternating streams: the latency-bound tail of chunk k (a few long-running CTAs, the
     # one-CTA-per-scan prefix kernel) overlaps the start of chunk k+1 instead of leaving the GPU half empty
     streams = _device_streams(up.dev)[1]
     d2h = _device_streams(up.dev)[3]          # to_host=True: the pixels of finished sub-batches go back on their own stream
     n_done = 0
+    n_files = 0
     # ONE worker thread prepares the sub-batches.  Two were tried, both as two whole-task workers and as a gather
     # thread feeding a planning thread: the gathers fight for host memory bandwidth, the Python halves for the GIL, and
     # the run-to-run spread (61..73 ms per 4096 files) ate the 1-2 ms the overlap gained.
@@ -216,8 +226,12 @@ def _stream(up, it, depth, device, keep_coefficients=False, to_host=False):
             raw_dev.record_stream(st)
             desc[0].record_stream(st)
             st.wait_event(ev_desc)
+            sc = scales
+            if callable(scales):                  # the images' sizes are known only now that the sub-batch is planned
+                sc = scales(plan.geom.images, np.arange(n_files, n_files + len(chunk_files)))
+            n_files += len(chunk_files)
             batch = decode_batch_on_device(None, device=device, packed=packed, plan=plan, check=False,
-                                           raw_dev=raw_dev, raw_ready=ev, desc=desc, stream=st)
+                                           raw_dev=raw_dev, raw_ready=ev, desc=desc, stream=st, scales=sc)
             pending.append((batch, chunk_files))
             if len(pending) >= _N_STREAMS:
                 b, fl = pending.pop(0)

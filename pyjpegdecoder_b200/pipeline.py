@@ -425,6 +425,7 @@ class _LazyViews:
     asked for (a 4096-image batch would otherwise spend tens of milliseconds making views nobody may look at)."""
 
     def __init__(self, geom, out: torch.Tensor):
+        """geom: anything with out_offsets / out_shapes (BatchGeometry, scaled.OutputLayout)."""
         self._g, self._out = geom, out
         self._cache: Dict[int, torch.Tensor] = {}
 
@@ -453,13 +454,25 @@ class _LazyViews:
 class DecodedBatch:
     """Result of decoding a batch on one device."""
 
-    def __init__(self, plan: BatchPlan, out: torch.Tensor, coef: torch.Tensor, err: torch.Tensor, stats: dict):
+    def __init__(self, plan: BatchPlan, out: torch.Tensor, coef: torch.Tensor, err: torch.Tensor, stats: dict,
+                 layout=None):
+        """layout: scaled.OutputLayout of `out` when the batch was decoded at reduced size (None: the planner's)."""
         self.plan = plan
         self.out = out
         self.coef = coef
         self.err = err
         self.stats = stats
-        self.images = _LazyViews(plan.geom, out)    # (H, W, 3) / (H, W) uint8 device tensors, made on first use
+        self._layout = layout
+        self.images = _LazyViews(layout if layout is not None else plan.geom, out)    # (H, W, 3) / (H, W) uint8 device
+                                                                                       # tensors, made on first use
+
+    @property
+    def layout(self):
+        """scaled.OutputLayout: where each image's pixels lie in `out` (offset, pitch, size, channels)."""
+        if self._layout is None:
+            from .scaled import OutputLayout
+            self._layout = OutputLayout.from_geometry(self.plan.geom)
+        return self._layout
 
     def image_array(self, i: int) -> torch.Tensor:
         """The reference's layout: (W, H, 3) or (W, H) view (jpeg_decoder.py:626, :1373-1386)."""
@@ -487,7 +500,7 @@ class DecodedBatch:
                 done = torch.cuda.Event()
                 done.record(cs)
         self._host, self._host_done = host, done
-        self._host_views = _LazyViews(self.plan.geom, host)
+        self._host_views = _LazyViews(self._layout if self._layout is not None else self.plan.geom, host)
 
     def host_image(self, i: int) -> Optional[np.ndarray]:
         """(H, W, 3) / (H, W) numpy view of image i in the pinned host copy (None if start_host_copy was not called)."""
@@ -601,6 +614,7 @@ class DevicePipeline:
                 self.blk_pos = (torch.empty(g.total_blocks, dtype=torch.int32, device=dev)
                                 if any(grp.mode == 4 for grp in plan.groups) else None)
                 self.out = None
+                self.layout = None
         self.B = EntropyBuffers(self.words.data_ptr(), self.words_len, self.stream_start.data_ptr(),
                                 self.stream_end.data_ptr(), self.stream_sub.data_ptr(), self.sub_entry.data_ptr(),
                                 self.sub_exit.data_ptr(), self.sub_count.data_ptr(), self.sub_prefix.data_ptr(),
@@ -620,10 +634,20 @@ class DevicePipeline:
         with torch.cuda.device(self.dev), torch.cuda.stream(self.stream):
             self.raw.copy_(raw_host, non_blocking=True)
 
-    def launch(self, out_kind: int = _native.OUT_RGB, upto_group: Optional[int] = None, events: Optional[dict] = None):
+    def launch(self, out_kind: int = _native.OUT_RGB, upto_group: Optional[int] = None, events: Optional[dict] = None,
+               scales=None):
         """Enqueue un-stuffing, entropy decode and the pixel kernel.  With `events` (a dict), CUDA events
-        are recorded around each stage: events[stage] = list of (start, end) pairs."""
+        are recorded around each stage: events[stage] = list of (start, end) pairs.
+        scales: None (full size), or one scale / per-image scales in (1, 2, 4, 8) for RGB output at reduced size
+        (scaled.launch); self.layout then describes the output."""
         L, plan, B = self.L, self.plan, self.B
+        if scales is not None:
+            from . import scaled
+            if out_kind != _native.OUT_RGB:
+                raise ValueError("a reduced-size decode gives RGB / grey output only")
+            scales = scaled.per_image(scales, len(plan.parsed))
+            if (scales == 1).all():
+                scales = None
         s = self.stream
         cs = s.cuda_stream
         n_launch = 0
@@ -672,21 +696,33 @@ class DevicePipeline:
                 else:
                     timed("other_scans", lambda: call(7))
                     n_launch += 2 if grp.mode == 4 else 1
-            if self.out is None or self._out_kind != out_kind:
-                self.out = None
-            holder = {}
+            if scales is not None:
+                holder = {}
 
-            def pix():
-                holder["out"] = run_pixels(self.dg, self.coef, _native.IN_COEF, out_kind, out=self.out, stream=s)
-            timed("pixels", pix)
-            self.out = holder["out"]
-            self._out_kind = out_kind
-            n_launch += 1
+                def pix_scaled():
+                    holder["out"], holder["layout"] = scaled.launch(self.dg, self.coef, scales, s)
+                timed("pixels", pix_scaled)
+                self.out, self.layout = holder["out"], holder["layout"]
+                self._out_kind = None                   # the next full-size launch allocates its own output
+                n_launch += int((scales > 1).any()) + int((scales == 1).any())
+            else:
+                if self.out is None or self._out_kind != out_kind:
+                    self.out = None
+                holder = {}
+
+                def pix():
+                    holder["out"] = run_pixels(self.dg, self.coef, _native.IN_COEF, out_kind, out=self.out, stream=s)
+                timed("pixels", pix)
+                self.out = holder["out"]
+                self._out_kind = out_kind
+                self.layout = None
+                n_launch += 1
         self.kernel_launches_per_step = n_launch
         return self.out
 
     def result(self) -> "DecodedBatch":
-        return DecodedBatch(self.plan, self.out, self.coef, self.err, {"sync_changes": self.sync_changes, "_pipe": self})
+        return DecodedBatch(self.plan, self.out, self.coef, self.err, {"sync_changes": self.sync_changes, "_pipe": self},
+                            layout=self.layout)
 
 
 def decode_batch_on_device(datas: Optional[Sequence[bytes]], device=None, parsed: Optional[Sequence[ParsedJpeg]] = None,
@@ -694,10 +730,12 @@ def decode_batch_on_device(datas: Optional[Sequence[bytes]], device=None, parsed
                            stream: Optional[torch.cuda.Stream] = None, upto_wave: Optional[int] = None,
                            plan: Optional[BatchPlan] = None, out_kind: int = _native.OUT_RGB,
                            raw_dev: Optional[torch.Tensor] = None, raw_ready: Optional[torch.cuda.Event] = None,
-                           desc=None) -> DecodedBatch:
+                           desc=None, scales=None) -> DecodedBatch:
     """Decode a batch of JPEG file images on one GPU.  Returns device tensors; with check=True the
     per-image error words are read back (one synchronisation) and turned into exceptions.
-    upto_wave=k stops the entropy stage after the first k scan groups (tests: per-scan parity)."""
+    upto_wave=k stops the entropy stage after the first k scan groups (tests: per-scan parity).
+    scales: None (full size), one scale or per-image scales in (1, 2, 4, 8), or a function of the planned batch's
+    bj_image records that returns them (DevicePipeline.launch)."""
     require_cuda(device)
     if packed is None:
         packed = pack_files(datas, reuse_slot="checkout" if check else None,
@@ -723,7 +761,9 @@ def decode_batch_on_device(datas: Optional[Sequence[bytes]], device=None, parsed
                 parsed = [parse_jpeg(d) for d in datas]
             plan = BatchPlan(parsed, offsets, raw_host.numel(), serial_scans=upto_wave is not None)
     pipe = DevicePipeline(plan, device, stream, raw=raw_dev, desc=desc)
-    pipe.launch(out_kind=out_kind, upto_group=upto_wave)
+    if callable(scales):
+        scales = scales(plan.geom.images)
+    pipe.launch(out_kind=out_kind, upto_group=upto_wave, scales=scales)
     res = pipe.result()
     if check:
         err = pipe.err.cpu().numpy()               # synchronises: the upload has long completed

@@ -170,18 +170,17 @@ class _Resizer:
         (None: its pixels are complete already)."""
         if not items:
             return
-        g = batch.plan.geom
+        lay = batch.layout                               # full size or scaled: where each decoded image lies
         idx = np.fromiter((i for i, _ in items), dtype=np.int64, count=len(items))
-        rec = g.images[idx]
-        W, H = rec["width"].astype(np.int64), rec["height"].astype(np.int64)
+        W, H = lay.widths[idx], lay.heights[idx]
         roi = self.roi
         if isinstance(roi, np.ndarray) and roi.ndim == 2:
             roi = roi[np.fromiter((s for _, s in items), dtype=np.int64, count=len(items))]
         boxes = pixel_boxes(roi, W, H, self.size)
         jobs = np.zeros(len(items), dtype=RESIZE_JOB_DTYPE)
-        jobs["src_offset"] = rec["out_offset"]
-        jobs["src_pitch"] = rec["out_pitch"]
-        jobs["channels"] = np.where(rec["ncomp"] == 3, 3, 1)
+        jobs["src_offset"] = lay.offsets[idx]
+        jobs["src_pitch"] = lay.pitches[idx]
+        jobs["channels"] = lay.channels[idx]
         jobs["x0"], jobs["y0"], jobs["x1"], jobs["y1"] = boxes[:, 0], boxes[:, 1], boxes[:, 2], boxes[:, 3]
         jobs["dst_index"] = [s for _, s in items]
         staged = torch.empty(jobs.nbytes, dtype=torch.uint8, pin_memory=True)
@@ -201,7 +200,8 @@ class _Resizer:
 
 
 def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtype=torch.float32, mean=None, std=None,
-                     channels_last: bool = False, device=None, chunk: Optional[int] = None, on_error: str = "raise"):
+                     channels_last: bool = False, device=None, chunk: Optional[int] = None, on_error: str = "raise",
+                     scale=1):
     """Decode `files` (paths or bytes, like decode_batch) into ONE device tensor of shape (N, 3, h, w), (h, w) = size.
 
     Each image's region `roi` is resized like torch.nn.functional.interpolate(mode="bilinear", antialias=True,
@@ -216,10 +216,15 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
                 through decode_stream, so device memory stays bounded whatever the number of files.
       on_error  "raise", or "return": returns (tensor, errors) with errors[i] None or the exception of file i, whose
                 slot is zero.
+      scale     1, 2, 4 or 8: the files are decoded at 1/scale of their size in the DCT domain (decode_batch(scale=))
+                and the roi is taken on the decoded image; "auto": per file the largest of these whose roi box is
+                still at least (h, w), so nothing is upscaled that the full decode would have downscaled.
     The caller's current stream is ordered after the work, so the tensor can be used right away."""
     from .decoder import BATCH_CHUNK
+    from .scaled import check_scale
     if on_error not in ("raise", "return"):
         raise ValueError("on_error must be 'raise' or 'return'")
+    scale = check_scale(scale, allow_auto=True)
     h, w = _check_size(size)
     a, b = _fold_norm(dtype, mean, std)
     files = list(files)
@@ -228,6 +233,9 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
     chunk = BATCH_CHUNK if chunk is None else int(chunk)
     if chunk < 1:
         raise ValueError("chunk must be positive")
+    scales = None if scale == 1 else scale
+    if scale == "auto":
+        scales = _AutoScales(roi, (h, w))
 
     from .stages import require_cuda
     dev = require_cuda(device)
@@ -246,11 +254,11 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
         # which the caller's stream must not reuse before they are done
         try:
             if on_error == "return":
-                return out, _tolerant(files, rs, dev, chunk, cur)
+                return out, _tolerant(files, rs, dev, chunk, cur, scales)
             if n > chunk + chunk // 2:
-                from .loader import decode_stream
+                from .loader import _decode_stream
                 slot = 0
-                for part in decode_stream(files, chunk=chunk, device=dev):
+                for part in _decode_stream(files, chunk, dev, scales=scales):
                     # decode_stream yields a sub-batch after synchronising the stream it was decoded on
                     batch = part[0]._batch
                     rs.resize(batch, [(i, slot + i) for i in range(len(part))], None)
@@ -258,7 +266,7 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
                     del part, batch                     # the sub-batch's RGB and work buffers go back to the allocator
             else:
                 from .decoder import decode_batch
-                part = decode_batch(files, device=dev, chunk=chunk)
+                part = decode_batch(files, device=dev, chunk=chunk, _scales=scales)
                 rs.resize(part[0]._batch, [(i, i) for i in range(n)], cur)
                 del part
         finally:
@@ -266,13 +274,30 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
     return out
 
 
-def _tolerant(files: list, rs: _Resizer, dev, chunk: int, cur) -> list:
+class _AutoScales:
+    """scale="auto" of decode_to_tensor as a function of a planned sub-batch: (bj_image records, indices of its files
+    among decode_to_tensor's files) -> per-image scales (scaled.auto_scales).  offset: added to the indices, for
+    sub-batches whose indices count from a later file."""
+
+    def __init__(self, roi, size, offset: int = 0):
+        self.roi, self.size, self.offset = roi, size, offset
+
+    def __call__(self, images, idx):
+        from .scaled import auto_scales
+        roi = self.roi
+        if isinstance(roi, np.ndarray) and roi.ndim == 2:
+            roi = roi[np.asarray(idx, dtype=np.int64) + self.offset]
+        return auto_scales(images["width"], images["height"], roi, self.size)
+
+
+def _tolerant(files: list, rs: _Resizer, dev, chunk: int, cur, scales=None) -> list:
     """on_error="return": decode_batch(on_error="return") chunk by chunk, each chunk's good images resized into their
     slots (bad slots keep the zeros the output was created with)."""
     from .decoder import decode_batch
     errors: list = [None] * len(files)
     for c0 in range(0, len(files), chunk):
-        res = decode_batch(files[c0:c0 + chunk], device=dev, chunk=chunk, on_error="return")
+        sc = _AutoScales(scales.roi, scales.size, c0) if isinstance(scales, _AutoScales) else scales
+        res = decode_batch(files[c0:c0 + chunk], device=dev, chunk=chunk, on_error="return", _scales=sc)
         groups = {}
         for k, r in enumerate(res):
             if isinstance(r, Exception):
