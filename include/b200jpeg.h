@@ -226,8 +226,8 @@ bj_status bj_entropy_decode(const bj_scan* scans, int scan_first, int n_scans, i
 #define BJ_IN_SAMPLES 1  /* sample buffer produced by BJ_OUT_SAMPLES */
 
 int bj_version(void);
-int bj_sizeof(int what);         /* 0: sizeof(bj_image), 1: sizeof(bj_resize_job), 2: sizeof(bj_scaled_job) -- lets a
-                                    binding verify its struct mirrors */
+int bj_sizeof(int what);         /* 0: sizeof(bj_image), 1: sizeof(bj_resize_job), 2: sizeof(bj_scaled_job),
+                                    3: sizeof(bj_crop_job) -- lets a binding verify its struct mirrors */
 int bj_sizeof_entropy(int what); /* 1: sizeof(bj_scan), 2: sizeof(bj_entropy_buffers), 3: BJ_SUBSEQ_BITS */
 int bj_pixels_fast_strip(int layout); /* MCUs per CTA the specialised pixel kernel uses for BJ_LAYOUT_* (0: generic) */
 const char* bj_last_cuda_error(void);
@@ -381,6 +381,44 @@ typedef struct bj_scaled_job {   /* 24 bytes */
  */
 bj_status bj_pixels_scaled(const bj_image* images, const bj_scaled_job* jobs, int n_jobs, int max_strips,
                            const int16_t* coef, const int16_t* qtabs, uint8_t* out, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Crop decode: only the MCUs under a pixel box, at scale 1, 2, 4 or 8 (nvJPEG's ROI decode, libjpeg-turbo's
+ * jpeg_crop_scanline).  The box [x0, x1) x [y0, y1) is in pixels of the image decoded at 1/s (s = 1 << log2_scale)
+ * and lies inside it: x0 < x1 <= ceil(W / s), y0 < y1 <= ceil(H / s).
+ * Window rule: with an MCU of mw = 8 hmax / s by mh = 8 vmax / s pixels at that scale, the job decodes the MCUs
+ * [x0 / mw, ceil(x1 / mw)) x [y0 / mh, ceil(y1 / mh)) -- every MCU the box touches, no other.  A full-size MCU's
+ * chroma interpolation and a scaled block's tile never read outside their own MCU, so the window's pixels are the
+ * bytes bj_pixels / bj_pixels_scaled would write there.
+ * Output contract: pixel (x, y) of the box goes to out + out_offset + (y - y0) * out_pitch + (x - x0) * channels; nothing
+ * else is written.  Rows may start at any byte address.
+ * ------------------------------------------------------------------------------------------- */
+typedef struct bj_crop_job {   /* 40 bytes */
+    uint64_t out_offset;       /* byte offset of box pixel (x0, y0) in out */
+    uint32_t out_pitch;        /* bytes per row, >= (x1 - x0) * channels */
+    uint32_t image;            /* index into images */
+    uint32_t log2_scale;       /* 0, 1, 2 or 3 */
+    uint32_t x0, y0, x1, y1;   /* the box, in pixels of the image decoded at 1/s */
+    uint32_t reserved;
+} bj_crop_job;
+
+#define BJ_CROP_SCALED 8       /* bit of bj_pixels_crop's `kinds`: some job has log2_scale > 0 */
+
+/*
+ *   images      DEVICE array of bj_image, the records bj_pixels reads; out_offset and out_pitch are not used
+ *   jobs        DEVICE array of n_jobs bj_crop_job: any mix of images, layouts and scales
+ *   max_strips  max over jobs of (window rows) * ceil((window columns) / S), S = the image's strip_mcus at s = 1 and
+ *               bj_pixels_scaled's MCUs per CTA at s > 1
+ *   coef, total_blocks, qtabs, idct_table_t, stats   as for bj_pixels (COEF in, RGB out)
+ *   out         uint8 pixels at each job's out_offset / out_pitch
+ *   kinds       which kernels have work: bit BJ_LAYOUT_* for the layouts of the jobs at s = 1, bit BJ_CROP_SCALED for
+ *               jobs at s > 1 (as bj_pixels' layout_mask, it saves the launches that would find no job)
+ * One call covers every job; each specialised layout keeps its own kernel (grid: strips of the job's MCU window x jobs;
+ * more than 65535 jobs are launched in slices).
+ */
+bj_status bj_pixels_crop(const bj_image* images, const bj_crop_job* jobs, int n_jobs, int max_strips,
+                         const int16_t* coef, uint64_t total_blocks, const int16_t* qtabs, const double* idct_table_t,
+                         uint8_t* out, uint32_t kinds, uint32_t* stats, void* stream);
 
 #ifdef __cplusplus
 }

@@ -22,6 +22,7 @@
 #include <stdio.h>
 
 #include "../../include/b200jpeg.h"
+#include "bj_crop.cuh"
 #include "bj_pixel_math.cuh"
 
 namespace {
@@ -226,26 +227,40 @@ __device__ __forceinline__ void pixel_run(Smem& sm, const bj_image& im, int out_
     s2[2] = make_uint2(bytes[4], bytes[5]);
 }
 
+// CROP: one CTA per strip of a bj_crop_job's MCU window (generic layout, scale 1, coefficients in, RGB out), storing
+// only the box; in_kind, out_kind and only_generic_layout are then ignored.
+template <bool CROP>
 __global__ void __launch_bounds__(kThreads, 3)
-bj_pixels_kernel(const bj_image* __restrict__ images, const void* __restrict__ in, int in_kind,
+bj_pixels_kernel(const bj_image* __restrict__ images, const void* __restrict__ in, int in_kind_arg,
                  const int16_t* __restrict__ qtabs, const double* __restrict__ tabT, void* __restrict__ out,
-                 int out_kind, int only_generic_layout, uint32_t* __restrict__ stats) {
+                 int out_kind_arg, int only_generic_layout, uint32_t* __restrict__ stats,
+                 const bj_crop_job* __restrict__ jobs) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
     __shared__ bj_image im;
+    const int in_kind = CROP ? BJ_IN_COEF : in_kind_arg;
+    const int out_kind = CROP ? BJ_OUT_RGB : out_kind_arg;
 
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
+    bj_crop_job jb{};
+    if constexpr (CROP) jb = jobs[blockIdx.y];
     {
-        const uint32_t* src = reinterpret_cast<const uint32_t*>(&images[blockIdx.y]);
+        const uint32_t* src = reinterpret_cast<const uint32_t*>(&images[CROP ? jb.image : blockIdx.y]);
         if (tid < (int)(sizeof(bj_image) / 4)) reinterpret_cast<uint32_t*>(&im)[tid] = src[tid];
     }
     __syncthreads();
-    if (only_generic_layout && im.layout != BJ_LAYOUT_GENERIC) return;  // handled by bj_pixels_fast.cu
-    const int strips_total = im.mcus_y * im.strips_per_row;
-    if ((int)blockIdx.x >= strips_total) return;
-    const int my = blockIdx.x / im.strips_per_row;
-    const int m0 = (blockIdx.x % im.strips_per_row) * im.strip_mcus;
-    const int M = min((int)im.strip_mcus, (int)im.mcus_x - m0);
+    int my, m0, M;
+    if constexpr (CROP) {
+        if (im.layout != BJ_LAYOUT_GENERIC || jb.log2_scale != 0) return;  // other kernels' jobs
+        if (!bj::crop_strip(jb, 8 * im.hmax, 8 * im.vmax, im.strip_mcus, blockIdx.x, my, m0, M)) return;
+    } else {
+        if (only_generic_layout && im.layout != BJ_LAYOUT_GENERIC) return;  // handled by bj_pixels_fast.cu
+        const int strips_total = im.mcus_y * im.strips_per_row;
+        if ((int)blockIdx.x >= strips_total) return;
+        my = blockIdx.x / im.strips_per_row;
+        m0 = (blockIdx.x % im.strips_per_row) * im.strip_mcus;
+        M = min((int)im.strip_mcus, (int)im.mcus_x - m0);
+    }
     const int bpm = im.blocks_per_mcu;
     const int nblk = M * bpm;
     const int64_t gblk0 = (int64_t)im.coef_block0 + ((int64_t)my * im.mcus_x + m0) * bpm;
@@ -397,12 +412,22 @@ bj_pixels_kernel(const bj_image* __restrict__ images, const void* __restrict__ i
         int r = pair / im.hmax, hx = pair % im.hmax;
         int m = (chunk << 5) + lane;
         if (r >= rows || m >= M) continue;
+        if constexpr (CROP) {
+            if (y0 + r < (int)jb.y0 || y0 + r >= (int)jb.y1) continue;   // rows outside the box are not stored
+        }
         if (hx) pixel_run<1>(sm, im, out_kind, m, m * bpm, r, row_stride_s, cols, out, gbase, stats);
         else pixel_run<0>(sm, im, out_kind, m, m * bpm, r, row_stride_s, cols, out, gbase, stats);
     }
     if (out_kind != BJ_OUT_RGB) return;
     __syncthreads();
 
+    if constexpr (CROP) {
+        int sx, sy, w, h;
+        uint8_t* g;
+        if (bj::crop_part(jb, x0, y0, cols, rows, ch, reinterpret_cast<uint8_t*>(out), sx, sy, w, h, g))
+            bj::crop_store(g, jb.out_pitch, sm.a + sy * row_stride_s, row_stride_s, sx * ch, w * ch, h, tid, kThreads);
+        return;
+    }
     // ---- coalesced copy-out of the staged rows -------------------------------------------------
     unsigned char* gout = reinterpret_cast<unsigned char*>(out) + gbase;
     const int nbytes = cols * ch;
@@ -438,7 +463,7 @@ extern "C" {
 int bj_version(void) { return BJ_VERSION; }
 int bj_sizeof(int what) {
     return what == 0 ? (int)sizeof(bj_image) : what == 1 ? (int)sizeof(bj_resize_job)
-         : what == 2 ? (int)sizeof(bj_scaled_job) : -1;
+         : what == 2 ? (int)sizeof(bj_scaled_job) : what == 3 ? (int)sizeof(bj_crop_job) : -1;
 }
 const char* bj_last_cuda_error(void) { return g_err; }
 
@@ -453,6 +478,15 @@ bj_status bj_pixels_fast_launch(const bj_image* images, int n_images, int max_st
 bj_status bj_pixels_420_launch(const bj_image* images, int n_images, int max_strips, const int16_t* coef,
                                uint64_t total_blocks, const int16_t* qtabs, const double* tabT, uint8_t* out,
                                uint32_t* stats, void* stream);
+
+bj_status bj_pixels_fast_crop_launch(const bj_image* images, const bj_crop_job* jobs, int n_jobs, int max_strips,
+                                     const int16_t* coef, const int16_t* qtabs, const double* tabT, uint8_t* out,
+                                     uint32_t layout_mask, uint32_t* stats, void* stream);
+bj_status bj_pixels_420_crop_launch(const bj_image* images, const bj_crop_job* jobs, int n_jobs, int max_strips,
+                                    const int16_t* coef, uint64_t total_blocks, const int16_t* qtabs, const double* tabT,
+                                    uint8_t* out, uint32_t* stats, void* stream);
+bj_status bj_pixels_scaled_crop_launch(const bj_image* images, const bj_crop_job* jobs, int n_jobs, int max_strips,
+                                       const int16_t* coef, const int16_t* qtabs, uint8_t* out, void* stream);
 
 bj_status bj_pixels(const bj_image* images, int n_images, int max_strips, const void* in, int in_kind,
                     uint64_t total_blocks, const int16_t* qtabs, const double* idct_table_t, void* out, int out_kind,
@@ -486,13 +520,48 @@ bj_status bj_pixels(const bj_image* images, int n_images, int max_strips, const 
         if (!(layout_mask & 1u)) return BJ_OK;
         only_generic = 1;
     }
-    cudaError_t e = cudaFuncSetAttribute(bj_pixels_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+    cudaError_t e = cudaFuncSetAttribute(bj_pixels_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
     if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels/attr");
     dim3 grid((unsigned)max_strips, (unsigned)n_images);
-    bj_pixels_kernel<<<grid, kThreads, sizeof(Smem), (cudaStream_t)stream>>>(images, in, in_kind, qtabs, idct_table_t, out,
-                                                                           out_kind, only_generic, stats);
+    bj_pixels_kernel<false><<<grid, kThreads, sizeof(Smem), (cudaStream_t)stream>>>(images, in, in_kind, qtabs, idct_table_t, out,
+                                                                                  out_kind, only_generic, stats, nullptr);
     e = cudaGetLastError();
     if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels/launch");
+    return BJ_OK;
+}
+
+bj_status bj_pixels_crop(const bj_image* images, const bj_crop_job* jobs, int n_jobs, int max_strips, const int16_t* coef,
+                         uint64_t total_blocks, const int16_t* qtabs, const double* idct_table_t, uint8_t* out,
+                         uint32_t kinds, uint32_t* stats, void* stream) {
+    static_assert(sizeof(bj_crop_job) == 40, "bj_crop_job layout");
+    if (!images || !jobs || n_jobs <= 0 || max_strips <= 0 || !coef || !qtabs || !idct_table_t || !out) return BJ_E_ARG;
+    if (n_jobs > 65535) {
+        // the job index rides on grid.y: larger batches run as slices (jobs hold absolute offsets)
+        for (int j0 = 0; j0 < n_jobs; j0 += 65535) {
+            const int n = n_jobs - j0 < 65535 ? n_jobs - j0 : 65535;
+            bj_status st = bj_pixels_crop(images, jobs + j0, n, max_strips, coef, total_blocks, qtabs, idct_table_t, out,
+                                          kinds, stats, stream);
+            if (st != BJ_OK) return st;
+        }
+        return BJ_OK;
+    }
+    bj_status st = BJ_OK;
+    if (kinds & (1u << BJ_LAYOUT_420))
+        st = bj_pixels_420_crop_launch(images, jobs, n_jobs, max_strips, coef, total_blocks, qtabs, idct_table_t, out,
+                                       stats, stream);
+    const uint32_t fast = kinds & ((1u << BJ_LAYOUT_422) | (1u << BJ_LAYOUT_440) | (1u << BJ_LAYOUT_444) | (1u << BJ_LAYOUT_GRAY));
+    if (st == BJ_OK && fast)
+        st = bj_pixels_fast_crop_launch(images, jobs, n_jobs, max_strips, coef, qtabs, idct_table_t, out, fast, stats,
+                                        stream);
+    if (st == BJ_OK && (kinds & BJ_CROP_SCALED))
+        st = bj_pixels_scaled_crop_launch(images, jobs, n_jobs, max_strips, coef, qtabs, out, stream);
+    if (st != BJ_OK || !(kinds & (1u << BJ_LAYOUT_GENERIC))) return st;
+    cudaError_t e = cudaFuncSetAttribute(bj_pixels_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)sizeof(Smem));
+    if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels_crop/attr");
+    bj_pixels_kernel<true><<<dim3((unsigned)max_strips, (unsigned)n_jobs), kThreads, sizeof(Smem), (cudaStream_t)stream>>>(
+        images, coef, BJ_IN_COEF, qtabs, idct_table_t, out, BJ_OUT_RGB, 1, stats, jobs);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels_crop/launch");
     return BJ_OK;
 }
 

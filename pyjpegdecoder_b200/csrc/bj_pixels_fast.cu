@@ -22,6 +22,7 @@
 #include <stdint.h>
 
 #include "../../include/b200jpeg.h"
+#include "bj_crop.cuh"
 #include "bj_pixel_math.cuh"
 
 extern "C" bj_status bj_set_cuda_error(cudaError_t e, const char* where);
@@ -370,11 +371,12 @@ __device__ __forceinline__ void pixel_run(const Tiles<L>& t, int m, int r, int h
     s2[2] = make_uint2(o[4], o[5]);
 }
 
-template <int HMAX, int VMAX, int NCOMP, int LAYOUT>
+// CROP: one CTA per strip of a bj_crop_job's MCU window (jobs of this layout at scale 1), storing only the box.
+template <int HMAX, int VMAX, int NCOMP, int LAYOUT, bool CROP>
 __global__ void __launch_bounds__(kThreads, 3)
 bj_pixels_fast_kernel(const bj_image* __restrict__ images, const int16_t* __restrict__ coef,
                       const int16_t* __restrict__ qtabs, const double* __restrict__ tabT,
-                      uint8_t* __restrict__ out, uint32_t* __restrict__ stats) {
+                      uint8_t* __restrict__ out, uint32_t* __restrict__ stats, const bj_crop_job* __restrict__ jobs) {
     using L = Lay<HMAX, VMAX, NCOMP>;
     extern __shared__ __align__(16) unsigned char smem[];
     __shared__ bj_image im;
@@ -382,22 +384,34 @@ bj_pixels_fast_kernel(const bj_image* __restrict__ images, const int16_t* __rest
     // The descriptor goes to shared memory for later use (visible after the barrier below); what the prologue needs
     // is read straight from global memory by every thread (one broadcast transaction each), which saves a barrier
     // and a shared-memory round trip in front of the tile request.
-    const bj_image* const gi = &images[blockIdx.y];
+    bj_crop_job jb{};
+    if constexpr (CROP) jb = jobs[blockIdx.y];
+    const bj_image* const gi = &images[CROP ? jb.image : blockIdx.y];
     {
         const uint32_t* src = reinterpret_cast<const uint32_t*>(gi);
         if (tid < (int)(sizeof(bj_image) / 4)) reinterpret_cast<uint32_t*>(&im)[tid] = src[tid];
     }
     if ((int)__ldg(&gi->layout) != LAYOUT) return;
-    const int g_mcus_x = (int)__ldg(&gi->mcus_x), g_mcus_y = (int)__ldg(&gi->mcus_y);
-    const int strips_per_row = (g_mcus_x + L::STRIP - 1) / L::STRIP;
-    if ((int)blockIdx.x >= g_mcus_y * strips_per_row) return;
+    const int g_mcus_x = (int)__ldg(&gi->mcus_x);
+    int my, m0, M;
+    if constexpr (CROP) {
+        if (jb.log2_scale != 0) return;
+        int sm0, sM;
+        if (!bj::crop_strip(jb, L::MCU_W, L::MCU_H, L::STRIP, blockIdx.x, my, sm0, sM)) return;
+        m0 = sm0 + warp * L::MPW;
+        M = min(L::MPW, sm0 + sM - m0);
+    } else {
+        const int g_mcus_y = (int)__ldg(&gi->mcus_y);
+        const int strips_per_row = (g_mcus_x + L::STRIP - 1) / L::STRIP;
+        if ((int)blockIdx.x >= g_mcus_y * strips_per_row) return;
+        my = blockIdx.x / strips_per_row;
+        m0 = (blockIdx.x - my * strips_per_row) * L::STRIP + warp * L::MPW;
+        M = min(L::MPW, g_mcus_x - m0);
+    }
 
     // ---- this warp's tile: requested first, so that the table set-up below runs while it is in flight -------
     float4* wtab = reinterpret_cast<float4*>(smem + kWarps * L::WARP_BYTES);
     int16_t* qt = reinterpret_cast<int16_t*>(smem + kWarps * L::WARP_BYTES + L::W_BYTES);
-    const int my = blockIdx.x / strips_per_row;
-    const int m0 = (blockIdx.x - my * strips_per_row) * L::STRIP + warp * L::MPW;
-    const int M = min(L::MPW, g_mcus_x - m0);
     Tiles<L> t;
     t.a = smem + warp * L::WARP_BYTES;
     t.b = t.a + L::A_BYTES;
@@ -510,7 +524,9 @@ bj_pixels_fast_kernel(const bj_image* __restrict__ images, const int16_t* __rest
         for (int u0 = 0; u0 < nunits; u0 += 32) {
             const int u = u0 + lane;
             const int m = u / (L::MCU_H * L::HMAX);
-            if (u < nunits && r < rows) {
+            bool row_ok = r < rows;
+            if constexpr (CROP) row_ok = row_ok && y0 + r >= (int)jb.y0 && y0 + r < (int)jb.y1;   // rows outside the box are not stored
+            if (u < nunits && row_ok) {
                 const bool wide = ((wide_mask >> (m * L::BPM)) & ((1u << L::BPM) - 1u)) != 0u;
                 pixel_run<L>(t, m, r, hx, ww, wide, stats);
             }
@@ -519,6 +535,13 @@ bj_pixels_fast_kernel(const bj_image* __restrict__ images, const int16_t* __rest
     __syncwarp();
 
     // ---- store this warp's rows -------------------------------------------------------------------------
+    if constexpr (CROP) {
+        int sx, sy, w, h;
+        uint8_t* g;
+        if (bj::crop_part(jb, x0, y0, cols, rows, L::CH, out, sx, sy, w, h, g))
+            bj::crop_store(g, jb.out_pitch, t.a + sy * L::ROW_BYTES, L::ROW_BYTES, sx * L::CH, w * L::CH, h, lane, 32);
+        return;
+    }
     uint8_t* gout = out + (int64_t)im.out_offset + (int64_t)y0 * im.out_pitch + (int64_t)x0 * L::CH;
     const int nbytes = cols * L::CH;
     const bool aligned = ((reinterpret_cast<uintptr_t>(gout) & 15) == 0) && ((im.out_pitch & 15) == 0);
@@ -547,14 +570,15 @@ bj_pixels_fast_kernel(const bj_image* __restrict__ images, const int16_t* __rest
     }
 }
 
-template <int HMAX, int VMAX, int NCOMP, int LAYOUT>
+// n_images: grid.y, the images (jobs == nullptr) or the crop jobs
+template <int HMAX, int VMAX, int NCOMP, int LAYOUT, bool CROP = false>
 cudaError_t launch(const bj_image* images, int n_images, int max_strips, const int16_t* coef, const int16_t* qtabs,
-                   const double* tabT, uint8_t* out, uint32_t* stats, cudaStream_t st) {
+                   const double* tabT, uint8_t* out, uint32_t* stats, cudaStream_t st, const bj_crop_job* jobs = nullptr) {
     using L = Lay<HMAX, VMAX, NCOMP>;
-    auto k = bj_pixels_fast_kernel<HMAX, VMAX, NCOMP, LAYOUT>;
+    auto k = bj_pixels_fast_kernel<HMAX, VMAX, NCOMP, LAYOUT, CROP>;
     cudaError_t e = cudaFuncSetAttribute(k, cudaFuncAttributeMaxDynamicSharedMemorySize, L::SMEM);
     if (e != cudaSuccess) return e;
-    k<<<dim3((unsigned)max_strips, (unsigned)n_images), kThreads, L::SMEM, st>>>(images, coef, qtabs, tabT, out, stats);
+    k<<<dim3((unsigned)max_strips, (unsigned)n_images), kThreads, L::SMEM, st>>>(images, coef, qtabs, tabT, out, stats, jobs);
     return cudaGetLastError();
 }
 
@@ -591,5 +615,24 @@ extern "C" bj_status bj_pixels_fast_launch(const bj_image* images, int n_images,
     if (e == cudaSuccess && (layout_mask & (1u << BJ_LAYOUT_GRAY)))
         e = launch<1, 1, 1, BJ_LAYOUT_GRAY>(images, n_images, max_strips, coef, qtabs, tabT, out, stats, st);
     if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels/fast");
+    return BJ_OK;
+}
+
+// Crop jobs (bj_pixels_crop) of the specialised layouts in layout_mask other than 4:2:0 (bj_pixels_mma.cu).
+extern "C" bj_status bj_pixels_fast_crop_launch(const bj_image* images, const bj_crop_job* jobs, int n_jobs,
+                                                int max_strips, const int16_t* coef, const int16_t* qtabs,
+                                                const double* tabT, uint8_t* out, uint32_t layout_mask,
+                                                uint32_t* stats, void* stream) {
+    cudaStream_t st = (cudaStream_t)stream;
+    cudaError_t e = cudaSuccess;
+    if (e == cudaSuccess && (layout_mask & (1u << BJ_LAYOUT_422)))
+        e = launch<2, 1, 3, BJ_LAYOUT_422, true>(images, n_jobs, max_strips, coef, qtabs, tabT, out, stats, st, jobs);
+    if (e == cudaSuccess && (layout_mask & (1u << BJ_LAYOUT_440)))
+        e = launch<1, 2, 3, BJ_LAYOUT_440, true>(images, n_jobs, max_strips, coef, qtabs, tabT, out, stats, st, jobs);
+    if (e == cudaSuccess && (layout_mask & (1u << BJ_LAYOUT_444)))
+        e = launch<1, 1, 3, BJ_LAYOUT_444, true>(images, n_jobs, max_strips, coef, qtabs, tabT, out, stats, st, jobs);
+    if (e == cudaSuccess && (layout_mask & (1u << BJ_LAYOUT_GRAY)))
+        e = launch<1, 1, 1, BJ_LAYOUT_GRAY, true>(images, n_jobs, max_strips, coef, qtabs, tabT, out, stats, st, jobs);
+    if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels_crop/fast");
     return BJ_OK;
 }

@@ -27,6 +27,7 @@
 #include <stdint.h>
 
 #include "../../include/b200jpeg.h"
+#include "bj_crop.cuh"
 #include "bj_pixel_math.cuh"
 
 extern "C" bj_status bj_set_cuda_error(cudaError_t e, const char* where);
@@ -469,22 +470,34 @@ __device__ __noinline__ BlockResult block_dense(const Tiles t, int R, int m, int
 }
 
 // 96 registers x 160 threads x 4 CTAs = 61440 of the SM's 65536 registers; 50 KB of shared memory per CTA
+// CROP: one CTA per strip of a bj_crop_job's MCU window (4:2:0 jobs at scale 1), storing only the box.
+template <bool CROP>
 __global__ void __maxnreg__(96)
 bj_pixels_420_kernel(const __grid_constant__ CUtensorMap tmap, const bj_image* __restrict__ images,
                      const int16_t* __restrict__ qtabs, const double* __restrict__ tabT, uint8_t* __restrict__ out,
-                     uint32_t* __restrict__ stats) {
+                     uint32_t* __restrict__ stats, const bj_crop_job* __restrict__ jobs) {
     extern __shared__ __align__(1024) unsigned char smem_raw[];   // SWIZZLE_128B wants a 1024-byte aligned tile
     Tiles t;
     t.base = smem_raw;
     const int tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
-    const bj_image* const gi = &images[blockIdx.y];
+    // (the job is read again for the store rather than kept in registers through phase A and B; phase B computes
+    // every row of the strip, not only the box's: a row filter there costs registers the kernel does not have)
+    const bj_image* const gi = &images[CROP ? __ldg(&jobs[blockIdx.y].image) : blockIdx.y];
     if ((int)__ldg(&gi->layout) != BJ_LAYOUT_420) return;
-    const int mcus_x = (int)__ldg(&gi->mcus_x), mcus_y = (int)__ldg(&gi->mcus_y);
-    const int strips_per_row = (mcus_x + kMcus - 1) / kMcus;
-    if ((int)blockIdx.x >= mcus_y * strips_per_row) return;
-    const int my = blockIdx.x / strips_per_row;
-    const int m0 = (blockIdx.x - my * strips_per_row) * kMcus;
-    const int M = min(kMcus, mcus_x - m0);
+    const int mcus_x = (int)__ldg(&gi->mcus_x);
+    int my, m0, M;
+    if constexpr (CROP) {
+        const bj_crop_job jb = jobs[blockIdx.y];
+        if (jb.log2_scale != 0) return;
+        if (!bj::crop_strip(jb, 16, 16, kMcus, blockIdx.x, my, m0, M)) return;
+    } else {
+        const int mcus_y = (int)__ldg(&gi->mcus_y);
+        const int strips_per_row = (mcus_x + kMcus - 1) / kMcus;
+        if ((int)blockIdx.x >= mcus_y * strips_per_row) return;
+        my = blockIdx.x / strips_per_row;
+        m0 = (blockIdx.x - my * strips_per_row) * kMcus;
+        M = min(kMcus, mcus_x - m0);
+    }
     Misc* misc = t.misc();
 
     // ---- prologue: one thread requests the coefficient tile and the weight fragments ------------------------------
@@ -660,6 +673,14 @@ bj_pixels_420_kernel(const __grid_constant__ CUtensorMap tmap, const bj_image* _
     __syncthreads();
 
     // ---- store the strip's rows ---------------------------------------------------------------------------------
+    if constexpr (CROP) {
+        const bj_crop_job jb = jobs[blockIdx.y];
+        int sx, sy, w, h;
+        uint8_t* g;
+        if (bj::crop_part(jb, x0, y0, cols, rows, 3, out, sx, sy, w, h, g))
+            bj::crop_store(g, jb.out_pitch, t.stage(sy), kRowBytes, sx * 3, w * 3, h, tid, kThreads);
+        return;
+    }
     const uint32_t pitch = __ldg(&gi->out_pitch);
     uint8_t* gout = out + (int64_t)__ldg(&gi->out_offset) + (int64_t)y0 * pitch + (int64_t)x0 * 3;
     const int nbytes = cols * 3;
@@ -706,10 +727,13 @@ EncodeTiledFn encode_tiled_fn() {
 
 extern "C" int bj_pixels_420_strip(void) { return kMcus; }
 
-// 4:2:0 images of the batch: coefficient buffer (total_blocks x 64 int16) -> RGB.
-extern "C" bj_status bj_pixels_420_launch(const bj_image* images, int n_images, int max_strips, const int16_t* coef,
-                                          uint64_t total_blocks, const int16_t* qtabs, const double* tabT, uint8_t* out,
-                                          uint32_t* stats, void* stream) {
+namespace {
+
+// grid.y = n_images (jobs == nullptr) or the crop jobs
+template <bool CROP>
+bj_status launch_420(const bj_image* images, const bj_crop_job* jobs, int n_images, int max_strips, const int16_t* coef,
+                     uint64_t total_blocks, const int16_t* qtabs, const double* tabT, uint8_t* out, uint32_t* stats,
+                     void* stream) {
     EncodeTiledFn enc = encode_tiled_fn();
     if (!enc) return bj_set_cuda_error(cudaErrorNotSupported, "bj_pixels/420: cuTensorMapEncodeTiled unavailable");
     if (total_blocks == 0 || total_blocks > 0x7fffffffull) return BJ_E_ARG;
@@ -722,13 +746,29 @@ extern "C" bj_status bj_pixels_420_launch(const bj_image* images, int n_images, 
                      CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                      CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) return bj_set_cuda_error(cudaErrorInvalidValue, "bj_pixels/420: cuTensorMapEncodeTiled");
-    cudaError_t e = cudaFuncSetAttribute(bj_pixels_420_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
+    cudaError_t e = cudaFuncSetAttribute(bj_pixels_420_kernel<CROP>, cudaFuncAttributeMaxDynamicSharedMemorySize, SMEM_BYTES);
     if (e == cudaSuccess)
-        e = cudaFuncSetAttribute(bj_pixels_420_kernel, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
+        e = cudaFuncSetAttribute(bj_pixels_420_kernel<CROP>, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared);
     if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels/420");
-    bj_pixels_420_kernel<<<dim3((unsigned)max_strips, (unsigned)n_images), kThreads, SMEM_BYTES, (cudaStream_t)stream>>>(
-        tmap, images, qtabs, tabT, out, stats);
+    bj_pixels_420_kernel<CROP><<<dim3((unsigned)max_strips, (unsigned)n_images), kThreads, SMEM_BYTES, (cudaStream_t)stream>>>(
+        tmap, images, qtabs, tabT, out, stats, jobs);
     e = cudaGetLastError();
     if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels/420");
     return BJ_OK;
+}
+
+}  // namespace
+
+// 4:2:0 images of the batch: coefficient buffer (total_blocks x 64 int16) -> RGB.
+extern "C" bj_status bj_pixels_420_launch(const bj_image* images, int n_images, int max_strips, const int16_t* coef,
+                                          uint64_t total_blocks, const int16_t* qtabs, const double* tabT, uint8_t* out,
+                                          uint32_t* stats, void* stream) {
+    return launch_420<false>(images, nullptr, n_images, max_strips, coef, total_blocks, qtabs, tabT, out, stats, stream);
+}
+
+// 4:2:0 crop jobs at scale 1 (bj_pixels_crop).
+extern "C" bj_status bj_pixels_420_crop_launch(const bj_image* images, const bj_crop_job* jobs, int n_jobs, int max_strips,
+                                               const int16_t* coef, uint64_t total_blocks, const int16_t* qtabs,
+                                               const double* tabT, uint8_t* out, uint32_t* stats, void* stream) {
+    return launch_420<true>(images, jobs, n_jobs, max_strips, coef, total_blocks, qtabs, tabT, out, stats, stream);
 }

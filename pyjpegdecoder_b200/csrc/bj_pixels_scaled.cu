@@ -14,7 +14,10 @@
 #include <cuda_runtime.h>
 #include <stdint.h>
 
+#include <type_traits>
+
 #include "../../include/b200jpeg.h"
+#include "bj_crop.cuh"
 #include "bj_scaled_math.cuh"
 
 extern "C" bj_status bj_set_cuda_error(cudaError_t e, const char* where);
@@ -45,14 +48,17 @@ __device__ __forceinline__ int scaled_strip_mcus(const bj_image& im) {
     return by_blocks < by_plane ? by_blocks : by_plane;
 }
 
+// Job = bj_crop_job: one CTA per strip of the job's MCU window, colour and store only for the box (bj_pixels_crop).
+template <class Job>
 __global__ void __launch_bounds__(kThreads, 3)
-bj_pixels_scaled_kernel(const bj_image* __restrict__ images, const bj_scaled_job* __restrict__ jobs,
+bj_pixels_scaled_kernel(const bj_image* __restrict__ images, const Job* __restrict__ jobs,
                         const int16_t* __restrict__ coef, const int16_t* __restrict__ qtabs, uint8_t* __restrict__ out) {
+    constexpr bool CROP = std::is_same<Job, bj_crop_job>::value;
     extern __shared__ __align__(16) unsigned char smem_raw[];
     Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
     __shared__ bj_image im;
     const int tid = threadIdx.x;
-    const bj_scaled_job jb = jobs[blockIdx.y];
+    const Job jb = jobs[blockIdx.y];
     {
         const uint32_t* src = reinterpret_cast<const uint32_t*>(&images[jb.image]);
         if (tid < (int)(sizeof(bj_image) / 4)) reinterpret_cast<uint32_t*>(&im)[tid] = src[tid];
@@ -61,11 +67,16 @@ bj_pixels_scaled_kernel(const bj_image* __restrict__ images, const bj_scaled_job
     const int l = (int)jb.log2_scale;
     if (l < 1 || l > 3) return;
     const int M_max = scaled_strip_mcus(im);
-    const int strips_per_row = ((int)im.mcus_x + M_max - 1) / M_max;
-    if ((int)blockIdx.x >= (int)im.mcus_y * strips_per_row) return;
-    const int my = blockIdx.x / strips_per_row;
-    const int m0 = (blockIdx.x - my * strips_per_row) * M_max;
-    const int M = min(M_max, (int)im.mcus_x - m0);
+    int my, m0, M;
+    if constexpr (CROP) {
+        if (!bj::crop_strip(jb, (8 * im.hmax) >> l, (8 * im.vmax) >> l, M_max, blockIdx.x, my, m0, M)) return;
+    } else {
+        const int strips_per_row = ((int)im.mcus_x + M_max - 1) / M_max;
+        if ((int)blockIdx.x >= (int)im.mcus_y * strips_per_row) return;
+        my = blockIdx.x / strips_per_row;
+        m0 = (blockIdx.x - my * strips_per_row) * M_max;
+        M = min(M_max, (int)im.mcus_x - m0);
+    }
     const int bpm = im.blocks_per_mcu;
     const int nblk = M * bpm;
     const int ch = im.ncomp == 3 ? 3 : 1;
@@ -131,9 +142,15 @@ bj_pixels_scaled_kernel(const bj_image* __restrict__ images, const bj_scaled_job
     // ---- colour into the staged rows ---------------------------------------------------------------------------------
     const int out_w = ((int)im.width + (1 << l) - 1) >> l, out_h = ((int)im.height + (1 << l) - 1) >> l;
     const int x0 = m0 * mcu_w, y0 = my * mcu_h;
-    const int cols = min(PC, out_w - x0), rows = min(mcu_h, out_h - y0);
+    int cols = min(PC, out_w - x0), rows = min(mcu_h, out_h - y0);
     if (cols <= 0 || rows <= 0) return;
-    uint8_t* gout = out + jb.out_offset + (int64_t)y0 * jb.out_pitch + (int64_t)x0 * ch;
+    int sx = 0, sy = 0;                                                 // first plane column / row that is stored
+    uint8_t* gout;
+    if constexpr (CROP) {
+        if (!bj::crop_part(jb, x0, y0, cols, rows, ch, out, sx, sy, cols, rows, gout)) return;
+    } else {
+        gout = out + jb.out_offset + (int64_t)y0 * jb.out_pitch + (int64_t)x0 * ch;
+    }
     const int nbytes = cols * ch;
     const int rs = ((nbytes + 15) & ~15) + 16;                          // staged row stride
     if (tid < rows) sm.lead[tid] = (int)(reinterpret_cast<uintptr_t>(gout + (int64_t)tid * jb.out_pitch) & 15);
@@ -141,7 +158,7 @@ bj_pixels_scaled_kernel(const bj_image* __restrict__ images, const bj_scaled_job
     const int plane = mcu_h * PC;
     for (int i = tid; i < rows * cols; i += kThreads) {
         const int r = i / cols, x = i - r * cols;
-        const float* P = &sm.p[r * PC + x];
+        const float* P = &sm.p[(r + sy) * PC + x + sx];
         unsigned char* d = sm.a + r * rs + sm.lead[r] + x * ch;
         if (ch == 3) {
             uint32_t R, G, B;
@@ -175,16 +192,30 @@ extern "C" bj_status bj_pixels_scaled(const bj_image* images, const bj_scaled_jo
                                       const int16_t* coef, const int16_t* qtabs, uint8_t* out, void* stream) {
     static_assert(sizeof(bj_scaled_job) == 24, "bj_scaled_job layout");
     if (!images || !jobs || n_jobs <= 0 || max_strips <= 0 || !coef || !qtabs || !out) return BJ_E_ARG;
-    cudaError_t e = cudaFuncSetAttribute(bj_pixels_scaled_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
+    cudaError_t e = cudaFuncSetAttribute(bj_pixels_scaled_kernel<bj_scaled_job>, cudaFuncAttributeMaxDynamicSharedMemorySize,
                                          (int)sizeof(Smem));
     if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels_scaled/attr");
     // the job index rides on grid.y (at most 65535): larger batches run as slices (jobs hold absolute offsets)
     for (int j0 = 0; j0 < n_jobs; j0 += 65535) {
         const int n = n_jobs - j0 < 65535 ? n_jobs - j0 : 65535;
-        bj_pixels_scaled_kernel<<<dim3((unsigned)max_strips, (unsigned)n), kThreads, sizeof(Smem), (cudaStream_t)stream>>>(
+        bj_pixels_scaled_kernel<bj_scaled_job><<<dim3((unsigned)max_strips, (unsigned)n), kThreads, sizeof(Smem), (cudaStream_t)stream>>>(
             images, jobs + j0, coef, qtabs, out);
         e = cudaGetLastError();
         if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels_scaled/launch");
     }
+    return BJ_OK;
+}
+
+// Crop jobs at s > 1 (bj_pixels_crop: n_jobs <= 65535; jobs at s = 1 are left to the full-size kernels).
+extern "C" bj_status bj_pixels_scaled_crop_launch(const bj_image* images, const bj_crop_job* jobs, int n_jobs,
+                                                  int max_strips, const int16_t* coef, const int16_t* qtabs, uint8_t* out,
+                                                  void* stream) {
+    cudaError_t e = cudaFuncSetAttribute(bj_pixels_scaled_kernel<bj_crop_job>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                                         (int)sizeof(Smem));
+    if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels_crop/scaled attr");
+    bj_pixels_scaled_kernel<bj_crop_job><<<dim3((unsigned)max_strips, (unsigned)n_jobs), kThreads, sizeof(Smem),
+                                           (cudaStream_t)stream>>>(images, jobs, coef, qtabs, out);
+    e = cudaGetLastError();
+    if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_pixels_crop/scaled launch");
     return BJ_OK;
 }

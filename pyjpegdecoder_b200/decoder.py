@@ -44,7 +44,8 @@ class JpegDecoder:
 
     def __init__(self, file: Union[str, Path, bytes], device: Optional[Union[str, torch.device]] = None,
                  verbose: bool = False, parsed: Optional[ParsedJpeg] = None, _batch: Optional[DecodedBatch] = None,
-                 _index: int = 0):
+                 _index: int = 0, scale: int = 1, crop=None):
+        """scale and crop as for decode_batch."""
         if isinstance(file, (bytes, bytearray, memoryview)):
             self.file_path = None
         else:
@@ -53,7 +54,11 @@ class JpegDecoder:
             data = _read(file)
             self.file_size = len(data)
             p = parsed if parsed is not None else parse_jpeg(data)
-            _batch = decode_batch_on_device([data], device=device, parsed=[p])
+            from .crop import check_crop
+            from .scaled import check_scale
+            scale, crop = check_scale(scale), check_crop(crop, 1)
+            _batch = decode_batch_on_device([data], device=device, parsed=[p], scales=None if scale == 1 else scale,
+                                            crops=None if crop is None else crop(None, [0]))
             _index = 0
         self._batch = _batch
         self._index = _index
@@ -191,7 +196,7 @@ BATCH_CHUNK = 512
 
 def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Union[str, torch.device]] = None,
                  chunk: Optional[int] = None, on_error: str = "raise", keep_coefficients: bool = False,
-                 to_host: bool = False, scale: int = 1, _scales=None) -> List[JpegDecoder]:
+                 to_host: bool = False, scale: int = 1, crop=None, _scales=None, _crops=None) -> List[JpegDecoder]:
     """Decode many files and return one JpegDecoder-like object per file (pixels stay on the device until
     `image_array` is read).  Small batches run as ONE device pipeline (one launch sequence for all files); batches
     larger than 1.5 x `chunk` files are cut into sub-batches of `chunk` files that flow through the streaming front
@@ -213,7 +218,14 @@ def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Unio
     scale=2, 4 or 8: every image is decoded at 1/scale of its size in the DCT domain, (ceil(H/s), ceil(W/s), 3), from
     the low-frequency corner of each block (csrc/bj_scaled_math.cuh); image_tensor, image_array, save() and DLPack give
     those pixels, image_width / image_height stay the file's.  _scales: per-image scales, or a function
-    (bj_image records of a sub-batch, indices of its files in `files`) -> scales (decode_to_tensor(scale="auto"))."""
+    (bj_image records of a sub-batch, indices of its files in `files`) -> scales (decode_to_tensor(scale="auto")).
+
+    crop=(x0, y0, x1, y1), one box for every file, or one box per file (a sequence or an (n, 4) integer array): only
+    the MCUs under each box are decoded (crop.py).  Boxes are half-open, in full-resolution pixels of the file, and
+    clipped to the image; at scale s the result is image_tensor[y0 // s:ceil(y1 / s), x0 // s:ceil(x1 / s)] of the
+    same-scale full decode, contiguous.  A box entirely outside its image is a ValueError for that file.  _crops: a
+    function like _scales that returns (n, 4) file boxes (decode_to_tensor(roi=))."""
+    from .crop import check_crop
     from .scaled import check_scale
     if on_error not in ("raise", "return"):
         raise ValueError("on_error must be 'raise' or 'return'")
@@ -221,20 +233,23 @@ def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Unio
     if _scales is None and scale != 1:
         _scales = scale
     files = list(files)
+    if _crops is None:
+        _crops = check_crop(crop, len(files))
     if not files:
         return []
     chunk = BATCH_CHUNK if chunk is None else int(chunk)
     if chunk < 1:
         raise ValueError("chunk must be positive")
     if on_error == "return":
-        return _decode_batch_tolerant(files, device, chunk, _scales)
+        return _decode_batch_tolerant(files, device, chunk, _scales, _crops)
     if len(files) > chunk + chunk // 2:
         from .loader import _decode_stream
         out: List[JpegDecoder] = []
-        for part in _decode_stream(files, chunk, device, keep_coefficients, to_host, _scales):
+        for part in _decode_stream(files, chunk, device, keep_coefficients, to_host, _scales, _crops):
             out.extend(part)
         return out
     scales = _for_files(_scales, np.arange(len(files)))
+    crops = _for_files(_crops, np.arange(len(files)))
     from .pipeline import FAST_PLAN_MIN_FILES
     if len(files) >= FAST_PLAN_MIN_FILES and all(isinstance(f, (str, Path)) for f in files):
         # paths: the C helper's threads read the files straight into the pinned staging buffer and walk them
@@ -246,26 +261,28 @@ def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Unio
         except Exception:
             release_pinned(raw)
             raise
-        batch = decode_batch_on_device(None, device=device, packed=(raw, offs), plan=plan, scales=scales)
+        batch = decode_batch_on_device(None, device=device, packed=(raw, offs), plan=plan, scales=scales, crops=crops)
     else:
         datas = [_read(f) for f in files]
-        batch = decode_batch_on_device(datas, device=device, scales=scales)
+        batch = decode_batch_on_device(datas, device=device, scales=scales, crops=crops)
     if to_host:
         batch.start_host_copy()
     return [JpegDecoder(f, _batch=batch, _index=i) for i, f in enumerate(files)]
 
 
 def _for_files(scales, idx: np.ndarray):
-    """decode_batch_on_device's scales for a sub-batch made of files[idx]: a function of (records, file indices) is
-    bound to the indices."""
+    """decode_batch_on_device's scales (or crops) for a sub-batch made of files[idx]: a function of (records, file
+    indices) is bound to the indices."""
     if callable(scales):
         return lambda images: scales(images, idx)
     return scales
 
 
-def _decode_batch_tolerant(files: list, device, chunk: int, scales=None) -> list:
+def _decode_batch_tolerant(files: list, device, chunk: int, scales=None, crops=None) -> list:
     """decode_batch(on_error="return"): header problems are found per file on the host (the same parser and plan
-    checks the batch path runs), entropy-data problems come back as the per-image device error words."""
+    checks the batch path runs), entropy-data problems come back as the per-image device error words.  A crop box
+    outside its image is that file's ValueError."""
+    from .crop import Boxes, outside, outside_error
     from .errors import JpegError
     from .pipeline import BatchPlan, error_for
     results: list = [None] * len(files)
@@ -274,16 +291,20 @@ def _decode_batch_tolerant(files: list, device, chunk: int, scales=None) -> list
     for i, f in enumerate(files):
         try:
             d = _read(f)
-            BatchPlan([parse_jpeg(d)], [0], len(d))          # header, scan script and size checks of one file
+            p = parse_jpeg(d)
+            BatchPlan([p], [0], len(d))                      # header, scan script and size checks of one file
         except JpegError as e:
             results[i] = e
+            continue
+        if isinstance(crops, Boxes) and outside(crops.box(i), p.width, p.height)[0]:
+            results[i] = outside_error(crops.box(i), p.width, p.height)
             continue
         datas[i] = d
         good.append(i)
     for a in range(0, len(good), chunk):
         idx = good[a:a + chunk]
         batch = decode_batch_on_device([datas[i] for i in idx], device=device, check=False,
-                                       scales=_for_files(scales, np.asarray(idx)))
+                                       scales=_for_files(scales, np.asarray(idx)), crops=_for_files(crops, np.asarray(idx)))
         pipe = batch.stats["_pipe"]
         err = pipe.err.cpu().numpy()                          # synchronises
         for k, i in enumerate(idx):

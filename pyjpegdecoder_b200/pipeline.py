@@ -456,7 +456,8 @@ class DecodedBatch:
 
     def __init__(self, plan: BatchPlan, out: torch.Tensor, coef: torch.Tensor, err: torch.Tensor, stats: dict,
                  layout=None):
-        """layout: scaled.OutputLayout of `out` when the batch was decoded at reduced size (None: the planner's)."""
+        """layout: scaled.OutputLayout of `out` when the batch was decoded at reduced size or cropped (None: the
+        planner's)."""
         self.plan = plan
         self.out = out
         self.coef = coef
@@ -635,13 +636,19 @@ class DevicePipeline:
             self.raw.copy_(raw_host, non_blocking=True)
 
     def launch(self, out_kind: int = _native.OUT_RGB, upto_group: Optional[int] = None, events: Optional[dict] = None,
-               scales=None):
+               scales=None, crops=None):
         """Enqueue un-stuffing, entropy decode and the pixel kernel.  With `events` (a dict), CUDA events
         are recorded around each stage: events[stage] = list of (start, end) pairs.
         scales: None (full size), or one scale / per-image scales in (1, 2, 4, 8) for RGB output at reduced size
-        (scaled.launch); self.layout then describes the output."""
+        (scaled.launch); self.layout then describes the output.
+        crops: None, or (n, 4) file boxes: only the pixels under each box are decoded, at the image's scale
+        (crop.launch); self.layout then describes the output."""
         L, plan, B = self.L, self.plan, self.B
-        if scales is not None:
+        if crops is not None:
+            from . import crop
+            if out_kind != _native.OUT_RGB:
+                raise ValueError("a crop decode gives RGB / grey output only")
+        elif scales is not None:
             from . import scaled
             if out_kind != _native.OUT_RGB:
                 raise ValueError("a reduced-size decode gives RGB / grey output only")
@@ -696,7 +703,17 @@ class DevicePipeline:
                 else:
                     timed("other_scans", lambda: call(7))
                     n_launch += 2 if grp.mode == 4 else 1
-            if scales is not None:
+            if crops is not None:
+                holder = {}
+
+                def pix_crop():
+                    holder["out"], holder["layout"] = crop.launch(self.dg, self.coef, 1 if scales is None else scales,
+                                                                  crops, s)
+                timed("pixels", pix_crop)
+                self.out, self.layout = holder["out"], holder["layout"]
+                self._out_kind = None                   # the next full-size launch allocates its own output
+                n_launch += 1
+            elif scales is not None:
                 holder = {}
 
                 def pix_scaled():
@@ -730,12 +747,14 @@ def decode_batch_on_device(datas: Optional[Sequence[bytes]], device=None, parsed
                            stream: Optional[torch.cuda.Stream] = None, upto_wave: Optional[int] = None,
                            plan: Optional[BatchPlan] = None, out_kind: int = _native.OUT_RGB,
                            raw_dev: Optional[torch.Tensor] = None, raw_ready: Optional[torch.cuda.Event] = None,
-                           desc=None, scales=None) -> DecodedBatch:
+                           desc=None, scales=None, crops=None) -> DecodedBatch:
     """Decode a batch of JPEG file images on one GPU.  Returns device tensors; with check=True the
     per-image error words are read back (one synchronisation) and turned into exceptions.
     upto_wave=k stops the entropy stage after the first k scan groups (tests: per-scan parity).
     scales: None (full size), one scale or per-image scales in (1, 2, 4, 8), or a function of the planned batch's
-    bj_image records that returns them (DevicePipeline.launch)."""
+    bj_image records that returns them (DevicePipeline.launch).
+    crops: None, one file box, (n, 4) file boxes, or a function of the planned batch's bj_image records that returns
+    them (crop.py); a box outside its image raises ValueError before anything is launched."""
     require_cuda(device)
     if packed is None:
         packed = pack_files(datas, reuse_slot="checkout" if check else None,
@@ -760,10 +779,13 @@ def decode_batch_on_device(datas: Optional[Sequence[bytes]], device=None, parsed
             if parsed is None:
                 parsed = [parse_jpeg(d) for d in datas]
             plan = BatchPlan(parsed, offsets, raw_host.numel(), serial_scans=upto_wave is not None)
+    if crops is not None:
+        from .crop import file_boxes
+        crops = file_boxes(crops, plan.geom.images)
     pipe = DevicePipeline(plan, device, stream, raw=raw_dev, desc=desc)
     if callable(scales):
         scales = scales(plan.geom.images)
-    pipe.launch(out_kind=out_kind, upto_group=upto_wave, scales=scales)
+    pipe.launch(out_kind=out_kind, upto_group=upto_wave, scales=scales, crops=crops)
     res = pipe.result()
     if check:
         err = pipe.err.cpu().numpy()               # synchronises: the upload has long completed

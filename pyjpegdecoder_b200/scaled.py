@@ -71,23 +71,33 @@ class OutputLayout:
     def scaled(cls, images: np.ndarray, scales: np.ndarray) -> "OutputLayout":
         """Images of the given bj_image records at per-image scales, back to back, every start 16-byte aligned."""
         s = np.asarray(scales, dtype=np.int64)
-        ch = np.where(images["ncomp"] == 3, 3, 1).astype(np.int64)
         w = -(-images["width"].astype(np.int64) // s)
         h = -(-images["height"].astype(np.int64) // s)
+        return cls.packed(w, h, np.where(images["ncomp"] == 3, 3, 1))
+
+    @classmethod
+    def packed(cls, widths, heights, channels) -> "OutputLayout":
+        """Images of the given sizes back to back, rows unpadded, every start 16-byte aligned."""
+        w, h = np.asarray(widths, dtype=np.int64), np.asarray(heights, dtype=np.int64)
+        ch = np.asarray(channels, dtype=np.int64)
         pitch = w * ch
         padded = (h * pitch + 15) & ~15
-        offsets = np.zeros(len(s), dtype=np.int64)
-        if len(s) > 1:
+        offsets = np.zeros(len(w), dtype=np.int64)
+        if len(w) > 1:
             np.cumsum(padded[:-1], out=offsets[1:])
         return cls(offsets, pitch, w, h, ch)
 
 
-def scaled_strips(images: np.ndarray) -> np.ndarray:
-    """CTAs of bj_pixels_scaled per image: mcus_y * ceil(mcus_x / MCUs per CTA)."""
+def scaled_strip_mcus(images: np.ndarray) -> np.ndarray:
+    """MCUs per CTA of bj_pixels_scaled per image."""
     bpm = images["blocks_per_mcu"].astype(np.int64)
     plane = images["ncomp"].astype(np.int64) * 16 * images["hmax"].astype(np.int64) * images["vmax"].astype(np.int64)
-    m = np.minimum(MAX_BLOCKS // bpm, PLANE // plane)
-    return images["mcus_y"].astype(np.int64) * -(-images["mcus_x"].astype(np.int64) // m)
+    return np.minimum(MAX_BLOCKS // bpm, PLANE // plane)
+
+
+def scaled_strips(images: np.ndarray) -> np.ndarray:
+    """CTAs of bj_pixels_scaled per image: mcus_y * ceil(mcus_x / MCUs per CTA)."""
+    return images["mcus_y"].astype(np.int64) * -(-images["mcus_x"].astype(np.int64) // scaled_strip_mcus(images))
 
 
 def auto_scales(widths, heights, roi, size) -> np.ndarray:
@@ -121,7 +131,7 @@ def _bind():
     return L
 
 
-def _upload(a: np.ndarray, device) -> torch.Tensor:
+def upload(a: np.ndarray, device) -> torch.Tensor:
     """Asynchronous copy of a small structured array on the current stream (the pinned block is kept by the
     allocator until the copy has completed)."""
     staged = torch.empty(a.nbytes, dtype=torch.uint8, pin_memory=True)
@@ -151,7 +161,7 @@ def launch(dg, coef: torch.Tensor, scales, stream: torch.cuda.Stream):
             jobs["image"] = big
             jobs["log2_scale"] = [_LOG2[int(s)] for s in sc[big]]
             max_strips = int(scaled_strips(rec[big]).max())
-            dev_jobs = _upload(jobs, dg.device)
+            dev_jobs = upload(jobs, dg.device)
             _native.check(L.bj_pixels_scaled(dg.images.data_ptr(), dev_jobs.data_ptr(), len(big), max_strips,
                                              coef.data_ptr(), dg.qtabs.data_ptr(), out.data_ptr(), stream.cuda_stream),
                           "bj_pixels_scaled")
@@ -163,7 +173,7 @@ def launch(dg, coef: torch.Tensor, scales, stream: torch.cuda.Stream):
             mask = 0
             for lv in np.unique(sub["layout"]):
                 mask |= 1 << int(lv)
-            dev_sub = _upload(sub, dg.device)
+            dev_sub = upload(sub, dg.device)
             _native.check(L.bj_pixels(dev_sub.data_ptr(), len(one), max_strips, coef.data_ptr(), _native.IN_COEF,
                                       g.total_blocks, dg.qtabs.data_ptr(), dg.table.data_ptr(), out.data_ptr(),
                                       _native.OUT_RGB, mask, None, stream.cuda_stream), "bj_pixels")

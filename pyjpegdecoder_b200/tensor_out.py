@@ -219,6 +219,8 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
       scale     1, 2, 4 or 8: the files are decoded at 1/scale of their size in the DCT domain (decode_batch(scale=))
                 and the roi is taken on the decoded image; "auto": per file the largest of these whose roi box is
                 still at least (h, w), so nothing is upscaled that the full decode would have downscaled.
+    With a roi, only each file's roi box is decoded (decode_batch(crop=)), taken at the scale the file uses; the
+    resize then reads the whole decoded crop, which holds the same bytes as the box of the full decode.
     The caller's current stream is ordered after the work, so the tensor can be used right away."""
     from .decoder import BATCH_CHUNK
     from .scaled import check_scale
@@ -236,6 +238,7 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
     scales = None if scale == 1 else scale
     if scale == "auto":
         scales = _AutoScales(roi, (h, w))
+    crops = None if roi is None else _RoiCrops(roi, (h, w), scales)
 
     from .stages import require_cuda
     dev = require_cuda(device)
@@ -248,17 +251,17 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
             out.zero_()
         if n == 0:
             return (out, []) if on_error == "return" else out
-        rs = _Resizer(out, roi, (h, w), dtype, a, b, channels_last)
+        rs = _Resizer(out, None if crops is not None else roi, (h, w), dtype, a, b, channels_last)
         cur = torch.cuda.current_stream(dev)
         # finish() also runs when a file raises part-way: resizes already enqueued may still be writing into `out`,
         # which the caller's stream must not reuse before they are done
         try:
             if on_error == "return":
-                return out, _tolerant(files, rs, dev, chunk, cur, scales)
+                return out, _tolerant(files, rs, dev, chunk, cur, scales, crops)
             if n > chunk + chunk // 2:
                 from .loader import _decode_stream
                 slot = 0
-                for part in _decode_stream(files, chunk, dev, scales=scales):
+                for part in _decode_stream(files, chunk, dev, scales=scales, crops=crops):
                     # decode_stream yields a sub-batch after synchronising the stream it was decoded on
                     batch = part[0]._batch
                     rs.resize(batch, [(i, slot + i) for i in range(len(part))], None)
@@ -266,7 +269,7 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
                     del part, batch                     # the sub-batch's RGB and work buffers go back to the allocator
             else:
                 from .decoder import decode_batch
-                part = decode_batch(files, device=dev, chunk=chunk, _scales=scales)
+                part = decode_batch(files, device=dev, chunk=chunk, _scales=scales, _crops=crops)
                 rs.resize(part[0]._batch, [(i, i) for i in range(n)], cur)
                 del part
         finally:
@@ -290,14 +293,37 @@ class _AutoScales:
         return auto_scales(images["width"], images["height"], roi, self.size)
 
 
-def _tolerant(files: list, rs: _Resizer, dev, chunk: int, cur, scales=None) -> list:
+class _RoiCrops:
+    """decode_to_tensor's roi as crop boxes of a planned sub-batch: (bj_image records, indices of its files among
+    decode_to_tensor's files) -> (n, 4) file boxes.  Each is the pixel_boxes box on the image decoded at the file's
+    scale s, times s, which decodes to exactly that box (crop.py's rule), so the resize sees today's box size and
+    bytes.  scales: None, one scale or a function like _AutoScales; offset as for _AutoScales."""
+
+    def __init__(self, roi, size, scales, offset: int = 0):
+        self.roi, self.size, self.scales, self.offset = roi, size, scales, offset
+
+    def __call__(self, images, idx):
+        n = len(idx)
+        if callable(self.scales):
+            s = np.asarray(self.scales(images, idx), dtype=np.int64)
+        else:
+            s = np.full(n, 1 if self.scales is None else self.scales, dtype=np.int64)
+        roi = self.roi
+        if isinstance(roi, np.ndarray) and roi.ndim == 2:
+            roi = roi[np.asarray(idx, dtype=np.int64) + self.offset]
+        W, H = images["width"].astype(np.int64), images["height"].astype(np.int64)
+        return pixel_boxes(roi, -(-W // s), -(-H // s), self.size) * s[:, None]
+
+
+def _tolerant(files: list, rs: _Resizer, dev, chunk: int, cur, scales=None, crops=None) -> list:
     """on_error="return": decode_batch(on_error="return") chunk by chunk, each chunk's good images resized into their
     slots (bad slots keep the zeros the output was created with)."""
     from .decoder import decode_batch
     errors: list = [None] * len(files)
     for c0 in range(0, len(files), chunk):
         sc = _AutoScales(scales.roi, scales.size, c0) if isinstance(scales, _AutoScales) else scales
-        res = decode_batch(files[c0:c0 + chunk], device=dev, chunk=chunk, on_error="return", _scales=sc)
+        cr = None if crops is None else _RoiCrops(crops.roi, crops.size, sc, c0)
+        res = decode_batch(files[c0:c0 + chunk], device=dev, chunk=chunk, on_error="return", _scales=sc, _crops=cr)
         groups = {}
         for k, r in enumerate(res):
             if isinstance(r, Exception):
