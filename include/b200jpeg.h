@@ -205,6 +205,10 @@ bj_status bj_entropy_plan(const bj_scan* scans, int scan_first, int n_scans, con
 #define BJ_PHASE_ALL 7
 #define BJ_PHASE_NO_BITMAP 8 /* testing: the chain step finds stream heads by binary search, the path it takes by
                                 itself for a scan of more than 262144 subsequences (128 MB of entropy-coded data) */
+#define BJ_PHASE_T81_REFINE 16 /* AC refinement corrections by the T.81 rule (G.1.2.3, libjpeg-turbo's): a correction bit
+                                  adds +-(1 << Al) by sign when that bit of the magnitude is clear, instead of the
+                                  reference's `coef |= 1 << Al` on the two's-complement value; DC refinement is the same
+                                  under both rules */
 bj_status bj_entropy_decode(const bj_scan* scans, int scan_first, int n_scans, int mode, uint32_t max_sub,
                             uint32_t max_streams, uint32_t max_blocks, uint32_t max_lut,
                             const bj_entropy_buffers* bufs, uint32_t* chain, int phases, void* stream);
@@ -419,6 +423,49 @@ typedef struct bj_crop_job {   /* 40 bytes */
 bj_status bj_pixels_crop(const bj_image* images, const bj_crop_job* jobs, int n_jobs, int max_strips,
                          const int16_t* coef, uint64_t total_blocks, const int16_t* qtabs, const double* idct_table_t,
                          uint8_t* out, uint32_t kinds, uint32_t* stats, void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * libjpeg-turbo-exact pixels (compat="libjpeg-turbo"): bit for bit what libjpeg-turbo's default jpeg_read_scanlines
+ * writes (JDCT_ISLOW, do_fancy_upsampling = TRUE, no merged upsampling; Pillow's Image.open pixels), from T.81
+ * coefficients (bj_entropy_decode with BJ_PHASE_T81_REFINE for progressive files).  Dequantisation as int (no int16
+ * wrap), jpeg_idct_islow with its range_limit table, jdsample.c's fancy upsampling -- which reads across MCU
+ * boundaries, with edges replicated at each component's real size ceil(W h / hmax) x ceil(H v / vmax) -- and jdcolor.c's
+ * table-exact YCbCr -> RGB.  The arithmetic is csrc/bj_ijg_math.cuh.  Full size only: jobs with log2_scale != 0 are
+ * skipped (nothing is written).
+ *
+ * Jobs are bj_crop_job: box [x0, x1) x [y0, y1) in pixels of the image, x0 < x1 <= W, y0 < y1 <= H; a full decode is
+ * one job with the box (0, 0, W, H) and the image's out_offset / out_pitch.
+ * Output contract: as bj_pixels_crop -- pixel (x, y) of the box goes to out + out_offset + (y - y0) * out_pitch +
+ * (x - x0) * channels, nothing else is written, rows may start at any byte.
+ * Halo rule (bj::ijg_window): a job decodes the MCUs its box touches, grown to every MCU that holds a sample the fancy
+ * upsampling of a box pixel reads: a component at ratio 2 in a direction (h2v1 / h2v2 with downsampled_width > 2, h1v2)
+ * reads sample j - 1 for the even pixel 2j (j > 0) and j + 1 for the odd pixel 2j + 1 (j below the last real sample), so
+ * the window grows by at most one MCU per side.  Call these MCUs [mx0, mx1) x [my0, my1).
+ * Workspace rule: `reserved` of each job holds the byte offset of its planes in `workspace` divided by 256; the
+ * job's planes are uint8, component after component, plane c having (mx1 - mx0) * 8 h_c columns and
+ * (my1 - my0) * 8 v_c rows, row-major without padding; jobs must not overlap.  The library allocates nothing: the
+ * caller sizes the workspace as the sum over jobs of these planes (each job's start rounded up to 256 bytes, see
+ * pyjpegdecoder_b200/ijg.py).
+ * ------------------------------------------------------------------------------------------- */
+#define BJ_IJG_IDCT 1          /* bit of bj_pixels_ijg's `kinds`: run the IDCT launch (coefficients -> planes) */
+#define BJ_IJG_COLOUR 2        /* run the upsample + colour launch (planes -> pixels) */
+#define BJ_IJG_ALL 3
+
+/*
+ *   images      DEVICE array of bj_image, the records bj_pixels reads; out_offset and out_pitch are not used
+ *   jobs        DEVICE array of n_jobs bj_crop_job: log2_scale 0, reserved = workspace offset / 256
+ *   max_strips  max over jobs of my1 - my0 (grid x of both launches: one CTA per MCU row of the window)
+ *   coef        coefficient buffer (zig-zag, quantised, T.81 refinement)
+ *   qtabs       as for bj_pixels
+ *   workspace   uint8 sample planes (workspace rule above), 256-byte aligned
+ *   out         uint8 pixels at each job's out_offset / out_pitch
+ *   kinds       BJ_IJG_ALL, or one of its two bits so that a caller can time the launches separately (the IDCT launch
+ *               must have run before the colour launch reads the planes)
+ * Returns BJ_E_ARG for a NULL buffer, n_jobs <= 0, max_strips <= 0 or a `kinds` outside BJ_IJG_ALL.
+ */
+bj_status bj_pixels_ijg(const bj_image* images, const bj_crop_job* jobs, int n_jobs, int max_strips,
+                        const int16_t* coef, const int16_t* qtabs, uint8_t* workspace, uint8_t* out, uint32_t kinds,
+                        void* stream);
 
 #ifdef __cplusplus
 }

@@ -849,6 +849,8 @@ __global__ void __launch_bounds__(32) acrefine_parse_kernel(const bj_scan* __res
     }
 }
 
+// T81: the T.81 correction rule (BJ_PHASE_T81_REFINE) instead of the reference's (acrefine_corrections)
+template <bool T81>
 __global__ void __launch_bounds__(128) acrefine_apply_kernel(const bj_scan* __restrict__ scans, int scan_first, bj_entropy_buffers B,
                                                              uint32_t lut_cap) {
     extern __shared__ __align__(16) unsigned char smem_raw[];
@@ -871,8 +873,8 @@ __global__ void __launch_bounds__(128) acrefine_apply_kernel(const bj_scan* __re
     const uint64_t mask = block_mask(v);
     const uint32_t end_rel = (uint32_t)(sb1 - sb0);
     uint32_t err;
-    if (sh.lut_in_smem) err = acrefine_block<true>(rd, sh.ctx, sh.lut + sh.ctx.ac_tab[0], end_rel, mask, eob_run, p);
-    else err = acrefine_block<true>(rd, sh.ctx, B.lut + sc.lut_off + sh.ctx.ac_tab[0], end_rel, mask, eob_run, p);
+    if (sh.lut_in_smem) err = acrefine_block<true, T81>(rd, sh.ctx, sh.lut + sh.ctx.ac_tab[0], end_rel, mask, eob_run, p);
+    else err = acrefine_block<true, T81>(rd, sh.ctx, B.lut + sc.lut_off + sh.ctx.ac_tab[0], end_rel, mask, eob_run, p);
     if (err) atomicOr(&B.err[sc.image], err);
 }
 
@@ -947,12 +949,16 @@ bj_status bj_entropy_decode(const bj_scan* scans, int scan_first, int n_scans, i
         const uint32_t win_bits = max_streams > 32u ? 4096u : (uint32_t)BJ_ACR_WIN_BITS;
         const size_t parse_smem = ((smem + 15) & ~(size_t)15) + sizeof(uint32_t) * win_bits;
         e = cudaFuncSetAttribute(acrefine_parse_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)parse_smem);
-        if (e == cudaSuccess) e = cudaFuncSetAttribute(acrefine_apply_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
+        const bool t81 = (phases & BJ_PHASE_T81_REFINE) != 0;
+        if (e == cudaSuccess)
+            e = cudaFuncSetAttribute(t81 ? acrefine_apply_kernel<true> : acrefine_apply_kernel<false>,
+                                     cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem);
         if (e != cudaSuccess) return bj_set_cuda_error(e, "bj_entropy_decode/attr");
         for (int s0 = 0; s0 < n_scans; s0 += 65535) {
             const int ns = n_scans - s0 < 65535 ? n_scans - s0 : 65535;
             acrefine_parse_kernel<<<dim3(max_streams, (unsigned)ns), 32, parse_smem, st>>>(scans, scan_first + s0, *bufs, lut_cap, win_bits);
-            acrefine_apply_kernel<<<dim3((max_blocks + 127) / 128, (unsigned)ns), 128, smem, st>>>(scans, scan_first + s0, *bufs, lut_cap);
+            if (t81) acrefine_apply_kernel<true><<<dim3((max_blocks + 127) / 128, (unsigned)ns), 128, smem, st>>>(scans, scan_first + s0, *bufs, lut_cap);
+            else acrefine_apply_kernel<false><<<dim3((max_blocks + 127) / 128, (unsigned)ns), 128, smem, st>>>(scans, scan_first + s0, *bufs, lut_cap);
         }
     } else {
         return BJ_E_ARG;

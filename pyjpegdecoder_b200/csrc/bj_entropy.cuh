@@ -402,6 +402,9 @@ BJ_HD uint32_t acfirst_run(BitReader<Src>& rd, int& z, const ScanCtx& c, const u
 //         and performs the stores -- fully parallel.
 // Correction is the reference's `coef |= bit << Al` on the two's-complement value (:1114), which is
 // NOT the T.81 rule for negative coefficients; bit-exact parity with the reference requires it.
+// T81 = true applies the T.81 rule instead (G.1.2.3, libjpeg-turbo's decode_mcu_AC_refine): a set bit adds
+// +-(1 << Al) by the coefficient's sign when that bit of its magnitude is still clear (compat="libjpeg-turbo").
+// Both rules keep every non-zero coefficient non-zero, so the non-zero masks and the parse are the same.
 BJ_HD int popc64(uint64_t x) {
 #if defined(__CUDA_ARCH__)
     return __popcll(x);
@@ -426,7 +429,7 @@ BJ_HD int nth_set64(uint64_t x, int n) {
 
 // The correction bits of the non-zero coefficients in `passed` (bit i = coefficient base + i), in
 // increasing zig-zag order (:1107-1115).
-template <bool APPLY, class Src>
+template <bool APPLY, bool T81 = false, class Src>
 BJ_HD void acrefine_corrections(BitReader<Src>& rd, uint64_t passed, int base, int16_t* p, int al) {
     int n = popc64(passed);
     if (!APPLY) {
@@ -439,7 +442,12 @@ BJ_HD void acrefine_corrections(BitReader<Src>& rd, uint64_t passed, int base, i
         for (int i = 0; i < k; i++) {
             const int zz = ctz64(passed);
             passed &= passed - 1;
-            if ((v << i) & 0x80000000u) p[base + zz] = (int16_t)(p[base + zz] | (int16_t)(1 << al));
+            if constexpr (T81) {
+                const int c = p[base + zz];
+                if (((v << i) & 0x80000000u) && !(c & (1 << al))) p[base + zz] = (int16_t)(c >= 0 ? c + (1 << al) : c - (1 << al));
+            } else {
+                if ((v << i) & 0x80000000u) p[base + zz] = (int16_t)(p[base + zz] | (int16_t)(1 << al));
+            }
         }
         rd.skip(k);
         n -= k;
@@ -449,7 +457,7 @@ BJ_HD void acrefine_corrections(BitReader<Src>& rd, uint64_t passed, int base, i
 // One block of an AC refinement stream.  m = non-zero history of the block (all 64 positions),
 // eob_run = blocks still covered by a running end-of-band run (0: the block starts with a symbol).
 // APPLY = false only advances the reader; APPLY = true also updates the block at p.
-template <bool APPLY, class Src>
+template <bool APPLY, bool T81 = false, class Src>
 BJ_HD uint32_t acrefine_block(BitReader<Src>& rd, const ScanCtx& c, const uint32_t* tab, uint32_t end_rel, uint64_t m,
                               uint32_t& eob_run, int16_t* p) {
     const int ss = c.ss, se = c.se, al = c.al;
@@ -477,7 +485,7 @@ BJ_HD uint32_t acrefine_block(BitReader<Src>& rd, const ScanCtx& c, const uint32
             const uint64_t zeros = ~rest & (~0ull >> z);
             const int idx = nth_set64(zeros, s ? r + 1 : 16);
             if (idx < 0) return BJ_ERR_COEF_INDEX;
-            acrefine_corrections<APPLY>(rd, rest & ((1ull << idx) - 1ull), z, p, al);
+            acrefine_corrections<APPLY, T81>(rd, rest & ((1ull << idx) - 1ull), z, p, al);
             if (APPLY && s) p[z + idx] = (int16_t)((uint32_t)newval << al);  // (:1225)
             z += idx + 1;
         }
@@ -486,7 +494,7 @@ BJ_HD uint32_t acrefine_block(BitReader<Src>& rd, const ScanCtx& c, const uint32
     // end-of-band run: the rest of this band (and the whole band of the blocks that follow inside the
     // run) only carries correction bits for its non-zero coefficients (:1258-1292)
     const uint64_t band = (~0ull << z) & (~0ull >> (63 - se));
-    acrefine_corrections<APPLY>(rd, m & band, 0, p, al);
+    acrefine_corrections<APPLY, T81>(rd, m & band, 0, p, al);
     eob_run--;
     return rd.rel > end_rel + 7 ? BJ_ERR_OVERRUN : 0u;
 }

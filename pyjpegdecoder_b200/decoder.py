@@ -44,8 +44,8 @@ class JpegDecoder:
 
     def __init__(self, file: Union[str, Path, bytes], device: Optional[Union[str, torch.device]] = None,
                  verbose: bool = False, parsed: Optional[ParsedJpeg] = None, _batch: Optional[DecodedBatch] = None,
-                 _index: int = 0, scale: int = 1, crop=None):
-        """scale and crop as for decode_batch."""
+                 _index: int = 0, scale: int = 1, crop=None, compat: str = "reference"):
+        """scale, crop and compat as for decode_batch."""
         if isinstance(file, (bytes, bytearray, memoryview)):
             self.file_path = None
         else:
@@ -55,10 +55,12 @@ class JpegDecoder:
             self.file_size = len(data)
             p = parsed if parsed is not None else parse_jpeg(data)
             from .crop import check_crop
+            from .ijg import check_compat
             from .scaled import check_scale
             scale, crop = check_scale(scale), check_crop(crop, 1)
+            check_compat(compat, scale)
             _batch = decode_batch_on_device([data], device=device, parsed=[p], scales=None if scale == 1 else scale,
-                                            crops=None if crop is None else crop(None, [0]))
+                                            crops=None if crop is None else crop(None, [0]), compat=compat)
             _index = 0
         self._batch = _batch
         self._index = _index
@@ -196,7 +198,8 @@ BATCH_CHUNK = 512
 
 def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Union[str, torch.device]] = None,
                  chunk: Optional[int] = None, on_error: str = "raise", keep_coefficients: bool = False,
-                 to_host: bool = False, scale: int = 1, crop=None, _scales=None, _crops=None) -> List[JpegDecoder]:
+                 to_host: bool = False, scale: int = 1, crop=None, compat: str = "reference", _scales=None,
+                 _crops=None) -> List[JpegDecoder]:
     """Decode many files and return one JpegDecoder-like object per file (pixels stay on the device until
     `image_array` is read).  Small batches run as ONE device pipeline (one launch sequence for all files); batches
     larger than 1.5 x `chunk` files are cut into sub-batches of `chunk` files that flow through the streaming front
@@ -224,12 +227,18 @@ def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Unio
     the MCUs under each box are decoded (crop.py).  Boxes are half-open, in full-resolution pixels of the file, and
     clipped to the image; at scale s the result is image_tensor[y0 // s:ceil(y1 / s), x0 // s:ceil(x1 / s)] of the
     same-scale full decode, contiguous.  A box entirely outside its image is a ValueError for that file.  _crops: a
-    function like _scales that returns (n, 4) file boxes (decode_to_tensor(roi=))."""
+    function like _scales that returns (n, 4) file boxes (decode_to_tensor(roi=)).
+
+    compat="reference" (default): the reference's pixels and coefficients.  compat="libjpeg-turbo": exactly what
+    libjpeg-turbo's default decompressor gives (ISLOW IDCT, fancy upsampling, its colour tables; Pillow's Image.open
+    pixels), and coefficient_planes() by the T.81 refinement rule; full size only (scale=1), with any crop (ijg.py)."""
     from .crop import check_crop
+    from .ijg import check_compat
     from .scaled import check_scale
     if on_error not in ("raise", "return"):
         raise ValueError("on_error must be 'raise' or 'return'")
     scale = check_scale(scale)
+    check_compat(compat, scale)
     if _scales is None and scale != 1:
         _scales = scale
     files = list(files)
@@ -241,11 +250,11 @@ def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Unio
     if chunk < 1:
         raise ValueError("chunk must be positive")
     if on_error == "return":
-        return _decode_batch_tolerant(files, device, chunk, _scales, _crops)
+        return _decode_batch_tolerant(files, device, chunk, _scales, _crops, compat)
     if len(files) > chunk + chunk // 2:
         from .loader import _decode_stream
         out: List[JpegDecoder] = []
-        for part in _decode_stream(files, chunk, device, keep_coefficients, to_host, _scales, _crops):
+        for part in _decode_stream(files, chunk, device, keep_coefficients, to_host, _scales, _crops, compat):
             out.extend(part)
         return out
     scales = _for_files(_scales, np.arange(len(files)))
@@ -261,10 +270,11 @@ def decode_batch(files: Sequence[Union[str, Path, bytes]], device: Optional[Unio
         except Exception:
             release_pinned(raw)
             raise
-        batch = decode_batch_on_device(None, device=device, packed=(raw, offs), plan=plan, scales=scales, crops=crops)
+        batch = decode_batch_on_device(None, device=device, packed=(raw, offs), plan=plan, scales=scales, crops=crops,
+                                       compat=compat)
     else:
         datas = [_read(f) for f in files]
-        batch = decode_batch_on_device(datas, device=device, scales=scales, crops=crops)
+        batch = decode_batch_on_device(datas, device=device, scales=scales, crops=crops, compat=compat)
     if to_host:
         batch.start_host_copy()
     return [JpegDecoder(f, _batch=batch, _index=i) for i, f in enumerate(files)]
@@ -278,7 +288,7 @@ def _for_files(scales, idx: np.ndarray):
     return scales
 
 
-def _decode_batch_tolerant(files: list, device, chunk: int, scales=None, crops=None) -> list:
+def _decode_batch_tolerant(files: list, device, chunk: int, scales=None, crops=None, compat: str = "reference") -> list:
     """decode_batch(on_error="return"): header problems are found per file on the host (the same parser and plan
     checks the batch path runs), entropy-data problems come back as the per-image device error words.  A crop box
     outside its image is that file's ValueError."""
@@ -304,7 +314,8 @@ def _decode_batch_tolerant(files: list, device, chunk: int, scales=None, crops=N
     for a in range(0, len(good), chunk):
         idx = good[a:a + chunk]
         batch = decode_batch_on_device([datas[i] for i in idx], device=device, check=False,
-                                       scales=_for_files(scales, np.asarray(idx)), crops=_for_files(crops, np.asarray(idx)))
+                                       scales=_for_files(scales, np.asarray(idx)), crops=_for_files(crops, np.asarray(idx)),
+                                       compat=compat)
         pipe = batch.stats["_pipe"]
         err = pipe.err.cpu().numpy()                          # synchronises
         for k, i in enumerate(idx):

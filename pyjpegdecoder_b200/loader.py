@@ -172,18 +172,21 @@ def _check(batch) -> None:
 
 def decode_stream(files: Iterable[Source], chunk: int = 512, device: Optional[Union[str, torch.device]] = None,
                   keep_coefficients: bool = False, to_host: bool = False, scale: int = 1,
-                  crop=None) -> Iterator[List[JpegDecoder]]:
+                  crop=None, compat: str = "reference") -> Iterator[List[JpegDecoder]]:
     """Decode an arbitrarily long sequence of files in sub-batches of at most `chunk` files (the first two are
     smaller, see _chunks); yields one list of JpegDecoder objects per sub-batch, in order.  Errors of a file (NotJpeg, CorruptedJpeg, ...) are raised when its chunk is reached.
     Three things overlap: the worker thread prepares and uploads the chunks ahead, the GPU decodes up to three chunks
     on alternating streams (a chunk is checked only when two later ones have been enqueued), and the caller consumes
     the oldest finished chunk.  scale=2, 4 or 8: reduced-size decode, as in decode_batch.  crop: one box, or one box
-    per file (`files` must then be sized), as in decode_batch."""
+    per file (`files` must then be sized), as in decode_batch.  compat: "reference" or "libjpeg-turbo", as in
+    decode_batch."""
     from .crop import check_crop
+    from .ijg import check_compat
     from .scaled import check_scale
     if chunk < 1:
         raise ValueError("chunk must be positive")
     scale = check_scale(scale)
+    check_compat(compat, scale)
     n = None
     if crop is not None:
         try:
@@ -191,10 +194,12 @@ def decode_stream(files: Iterable[Source], chunk: int = 512, device: Optional[Un
         except TypeError:
             n = None
     crops = check_crop(crop, n)
-    yield from _decode_stream(files, chunk, device, keep_coefficients, to_host, None if scale == 1 else scale, crops)
+    yield from _decode_stream(files, chunk, device, keep_coefficients, to_host, None if scale == 1 else scale, crops,
+                              compat)
 
 
-def _decode_stream(files, chunk, device, keep_coefficients=False, to_host=False, scales=None, crops=None):
+def _decode_stream(files, chunk, device, keep_coefficients=False, to_host=False, scales=None, crops=None,
+                   compat="reference"):
     """decode_stream with scales: None, one scale, or a function (bj_image records of a sub-batch, indices of its files
     in `files`) -> per-image scales, called once the sub-batch is planned; crops: None or such a function that returns
     (n, 4) file boxes."""
@@ -202,12 +207,12 @@ def _decode_stream(files, chunk, device, keep_coefficients=False, to_host=False,
     it = _chunks(files, chunk)
     depth = _N_SLOTS - 1                     # chunks prepared ahead of the one being enqueued
     try:
-        yield from _stream(up, it, depth, device, keep_coefficients, to_host, scales, crops)
+        yield from _stream(up, it, depth, device, keep_coefficients, to_host, scales, crops, compat)
     finally:
         up.close()
 
 
-def _stream(up, it, depth, device, keep_coefficients=False, to_host=False, scales=None, crops=None):
+def _stream(up, it, depth, device, keep_coefficients=False, to_host=False, scales=None, crops=None, compat="reference"):
     # consecutive chunks run on alternating streams: the latency-bound tail of chunk k (a few long-running CTAs, the
     # one-CTA-per-scan prefix kernel) overlaps the start of chunk k+1 instead of leaving the GPU half empty
     streams = _device_streams(up.dev)[1]
@@ -245,7 +250,8 @@ def _stream(up, it, depth, device, keep_coefficients=False, to_host=False, scale
                 cr = crops(plan.geom.images, idx)
             n_files += len(chunk_files)
             batch = decode_batch_on_device(None, device=device, packed=packed, plan=plan, check=False,
-                                           raw_dev=raw_dev, raw_ready=ev, desc=desc, stream=st, scales=sc, crops=cr)
+                                           raw_dev=raw_dev, raw_ready=ev, desc=desc, stream=st, scales=sc, crops=cr,
+                                           compat=compat)
             pending.append((batch, chunk_files))
             if len(pending) >= _N_STREAMS:
                 b, fl = pending.pop(0)

@@ -636,15 +636,25 @@ class DevicePipeline:
             self.raw.copy_(raw_host, non_blocking=True)
 
     def launch(self, out_kind: int = _native.OUT_RGB, upto_group: Optional[int] = None, events: Optional[dict] = None,
-               scales=None, crops=None):
+               scales=None, crops=None, compat: str = "reference"):
         """Enqueue un-stuffing, entropy decode and the pixel kernel.  With `events` (a dict), CUDA events
         are recorded around each stage: events[stage] = list of (start, end) pairs.
         scales: None (full size), or one scale / per-image scales in (1, 2, 4, 8) for RGB output at reduced size
         (scaled.launch); self.layout then describes the output.
         crops: None, or (n, 4) file boxes: only the pixels under each box are decoded, at the image's scale
-        (crop.launch); self.layout then describes the output."""
+        (crop.launch); self.layout then describes the output.
+        compat: "reference", or "libjpeg-turbo": T.81 AC refinement and libjpeg-turbo's pixels (ijg.launch, full size
+        only, with or without crops)."""
         L, plan, B = self.L, self.plan, self.B
-        if crops is not None:
+        from .ijg import PHASE_T81_REFINE, check_compat
+        ijg = check_compat(compat) == "libjpeg-turbo"
+        if ijg:
+            from .scaled import per_image
+            if out_kind != _native.OUT_RGB:
+                raise ValueError("a libjpeg-turbo decode gives RGB / grey output only")
+            if scales is not None and (per_image(scales, len(plan.parsed)) != 1).any():
+                check_compat(compat, scales)        # raises: full size only
+        elif crops is not None:
             from . import crop
             if out_kind != _native.OUT_RGB:
                 raise ValueError("a crop decode gives RGB / grey output only")
@@ -688,6 +698,8 @@ class DevicePipeline:
 
                 def call(phases, grp=grp):
                     phases |= self.extra_phase_flags
+                    if ijg and grp.mode == 4:
+                        phases |= PHASE_T81_REFINE
                     _native.check(L.bj_entropy_decode(
                         self.scans.data_ptr(), grp.first, grp.count, grp.mode, grp.max_sub, grp.max_streams,
                         grp.max_blocks, grp.max_lut, ctypes.byref(B), self.chain.data_ptr(), phases, cs),
@@ -703,7 +715,17 @@ class DevicePipeline:
                 else:
                     timed("other_scans", lambda: call(7))
                     n_launch += 2 if grp.mode == 4 else 1
-            if crops is not None:
+            if ijg:
+                from . import ijg as ijg_mod
+                holder = {}
+
+                def pix_ijg():
+                    holder["out"], holder["layout"] = ijg_mod.launch(self.dg, self.coef, crops, s)
+                timed("pixels", pix_ijg)
+                self.out, self.layout = holder["out"], holder["layout"]
+                self._out_kind = None                   # the next reference launch allocates its own output
+                n_launch += 2
+            elif crops is not None:
                 holder = {}
 
                 def pix_crop():
@@ -747,14 +769,15 @@ def decode_batch_on_device(datas: Optional[Sequence[bytes]], device=None, parsed
                            stream: Optional[torch.cuda.Stream] = None, upto_wave: Optional[int] = None,
                            plan: Optional[BatchPlan] = None, out_kind: int = _native.OUT_RGB,
                            raw_dev: Optional[torch.Tensor] = None, raw_ready: Optional[torch.cuda.Event] = None,
-                           desc=None, scales=None, crops=None) -> DecodedBatch:
+                           desc=None, scales=None, crops=None, compat: str = "reference") -> DecodedBatch:
     """Decode a batch of JPEG file images on one GPU.  Returns device tensors; with check=True the
     per-image error words are read back (one synchronisation) and turned into exceptions.
     upto_wave=k stops the entropy stage after the first k scan groups (tests: per-scan parity).
     scales: None (full size), one scale or per-image scales in (1, 2, 4, 8), or a function of the planned batch's
     bj_image records that returns them (DevicePipeline.launch).
     crops: None, one file box, (n, 4) file boxes, or a function of the planned batch's bj_image records that returns
-    them (crop.py); a box outside its image raises ValueError before anything is launched."""
+    them (crop.py); a box outside its image raises ValueError before anything is launched.
+    compat: "reference" or "libjpeg-turbo" (ijg.py; full size only)."""
     require_cuda(device)
     if packed is None:
         packed = pack_files(datas, reuse_slot="checkout" if check else None,
@@ -785,7 +808,7 @@ def decode_batch_on_device(datas: Optional[Sequence[bytes]], device=None, parsed
     pipe = DevicePipeline(plan, device, stream, raw=raw_dev, desc=desc)
     if callable(scales):
         scales = scales(plan.geom.images)
-    pipe.launch(out_kind=out_kind, upto_group=upto_wave, scales=scales, crops=crops)
+    pipe.launch(out_kind=out_kind, upto_group=upto_wave, scales=scales, crops=crops, compat=compat)
     res = pipe.result()
     if check:
         err = pipe.err.cpu().numpy()               # synchronises: the upload has long completed

@@ -201,7 +201,7 @@ class _Resizer:
 
 def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtype=torch.float32, mean=None, std=None,
                      channels_last: bool = False, device=None, chunk: Optional[int] = None, on_error: str = "raise",
-                     scale=1):
+                     scale=1, compat: str = "reference"):
     """Decode `files` (paths or bytes, like decode_batch) into ONE device tensor of shape (N, 3, h, w), (h, w) = size.
 
     Each image's region `roi` is resized like torch.nn.functional.interpolate(mode="bilinear", antialias=True,
@@ -219,6 +219,8 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
       scale     1, 2, 4 or 8: the files are decoded at 1/scale of their size in the DCT domain (decode_batch(scale=))
                 and the roi is taken on the decoded image; "auto": per file the largest of these whose roi box is
                 still at least (h, w), so nothing is upscaled that the full decode would have downscaled.
+      compat    "reference", or "libjpeg-turbo": the resize reads libjpeg-turbo's pixels (Pillow's), scale 1 only
+                (decode_batch(compat=)).
     With a roi, only each file's roi box is decoded (decode_batch(crop=)), taken at the scale the file uses; the
     resize then reads the whole decoded crop, which holds the same bytes as the box of the full decode.
     The caller's current stream is ordered after the work, so the tensor can be used right away."""
@@ -227,6 +229,8 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
     if on_error not in ("raise", "return"):
         raise ValueError("on_error must be 'raise' or 'return'")
     scale = check_scale(scale, allow_auto=True)
+    from .ijg import check_compat
+    check_compat(compat, scale)
     h, w = _check_size(size)
     a, b = _fold_norm(dtype, mean, std)
     files = list(files)
@@ -257,11 +261,11 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
         # which the caller's stream must not reuse before they are done
         try:
             if on_error == "return":
-                return out, _tolerant(files, rs, dev, chunk, cur, scales, crops)
+                return out, _tolerant(files, rs, dev, chunk, cur, scales, crops, compat)
             if n > chunk + chunk // 2:
                 from .loader import _decode_stream
                 slot = 0
-                for part in _decode_stream(files, chunk, dev, scales=scales, crops=crops):
+                for part in _decode_stream(files, chunk, dev, scales=scales, crops=crops, compat=compat):
                     # decode_stream yields a sub-batch after synchronising the stream it was decoded on
                     batch = part[0]._batch
                     rs.resize(batch, [(i, slot + i) for i in range(len(part))], None)
@@ -269,7 +273,7 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
                     del part, batch                     # the sub-batch's RGB and work buffers go back to the allocator
             else:
                 from .decoder import decode_batch
-                part = decode_batch(files, device=dev, chunk=chunk, _scales=scales, _crops=crops)
+                part = decode_batch(files, device=dev, chunk=chunk, compat=compat, _scales=scales, _crops=crops)
                 rs.resize(part[0]._batch, [(i, i) for i in range(n)], cur)
                 del part
         finally:
@@ -315,7 +319,7 @@ class _RoiCrops:
         return pixel_boxes(roi, -(-W // s), -(-H // s), self.size) * s[:, None]
 
 
-def _tolerant(files: list, rs: _Resizer, dev, chunk: int, cur, scales=None, crops=None) -> list:
+def _tolerant(files: list, rs: _Resizer, dev, chunk: int, cur, scales=None, crops=None, compat="reference") -> list:
     """on_error="return": decode_batch(on_error="return") chunk by chunk, each chunk's good images resized into their
     slots (bad slots keep the zeros the output was created with)."""
     from .decoder import decode_batch
@@ -323,7 +327,8 @@ def _tolerant(files: list, rs: _Resizer, dev, chunk: int, cur, scales=None, crop
     for c0 in range(0, len(files), chunk):
         sc = _AutoScales(scales.roi, scales.size, c0) if isinstance(scales, _AutoScales) else scales
         cr = None if crops is None else _RoiCrops(crops.roi, crops.size, sc, c0)
-        res = decode_batch(files[c0:c0 + chunk], device=dev, chunk=chunk, on_error="return", _scales=sc, _crops=cr)
+        res = decode_batch(files[c0:c0 + chunk], device=dev, chunk=chunk, on_error="return", compat=compat, _scales=sc,
+                           _crops=cr)
         groups = {}
         for k, r in enumerate(res):
             if isinstance(r, Exception):
