@@ -231,7 +231,8 @@ bj_status bj_entropy_decode(const bj_scan* scans, int scan_first, int n_scans, i
 
 int bj_version(void);
 int bj_sizeof(int what);         /* 0: sizeof(bj_image), 1: sizeof(bj_resize_job), 2: sizeof(bj_scaled_job),
-                                    3: sizeof(bj_crop_job) -- lets a binding verify its struct mirrors */
+                                    3: sizeof(bj_crop_job), 4: sizeof(bj_resize_pil_job) -- lets a binding verify its
+                                    struct mirrors */
 int bj_sizeof_entropy(int what); /* 1: sizeof(bj_scan), 2: sizeof(bj_entropy_buffers), 3: BJ_SUBSEQ_BITS */
 int bj_pixels_fast_strip(int layout); /* MCUs per CTA the specialised pixel kernel uses for BJ_LAYOUT_* (0: generic) */
 const char* bj_last_cuda_error(void);
@@ -354,6 +355,44 @@ typedef struct bj_resize_params {
  */
 bj_status bj_resize(const bj_resize_job* jobs, int n_jobs, const uint8_t* src, void* dst, const bj_resize_params* p,
                     void* stream);
+
+/* ---------------------------------------------------------------------------------------------
+ * Pillow's resample: PIL.Image.resize((VW, VH), BILINEAR | BICUBIC) of each job's source box, bit for bit, and of that
+ * virtual (VH, VW) image only the (out_h, out_w) window at (win_x, win_y) is computed -- torchvision's Resize(r) +
+ * CenterCrop(size) without the pixels the crop drops.  Arithmetic (csrc/bj_resize_pil_math.cuh): Resample.c's double
+ * coefficients rounded to 22-bit fixed point, the horizontal pass rounded to uint8, then the vertical pass; both
+ * in int32 (the header derives the bound).  Every output pixel uses the coefficients of the full (VW, VH) resize.
+ * Value of an output element of channel c: v * a[c] + b[c] in fp32, v the uint8 resampled value; uint8 output stores v
+ * (a = 1, b = 0 expected).  Greyscale sources give three channels (each with its a/b).
+ * ------------------------------------------------------------------------------------------- */
+#define BJ_PIL_BILINEAR 0
+#define BJ_PIL_BICUBIC 1
+
+typedef struct bj_resize_pil_job {   /* 56 bytes, 8-byte aligned */
+    uint64_t src_offset;   /* byte offset of pixel (0,0) in src; any alignment */
+    uint32_t src_pitch;    /* bytes per source row */
+    uint32_t channels;     /* 3 (RGB) or 1 (greyscale) */
+    uint32_t x0, y0, x1, y1; /* source box [x0, x1) x [y0, y1) in pixels: the image Pillow resizes */
+    uint32_t dst_index;    /* image slot n of the output tensor */
+    uint32_t virt_w, virt_h; /* the size the box is resized to, 1..2^31 - 1 (plain resize: out_w, out_h) */
+    uint32_t win_x, win_y; /* the window's offset in the virtual image, win_x + out_w <= virt_w, win_y + out_h <= virt_h
+                              (plain resize: 0, 0) */
+    uint32_t reserved;
+} bj_resize_pil_job;
+
+/*
+ *   jobs    DEVICE array of n_jobs bj_resize_pil_job
+ *   src     decoded uint8 pixels (bj_pixels' BJ_OUT_RGB buffer or any packed layout of the same form)
+ *   dst     output tensor storage, element type p->dtype, dense NCHW or NHWC
+ *   p       HOST pointer, as for bj_resize: out_h / out_w are the window's size
+ *   filter  BJ_PIL_BILINEAR or BJ_PIL_BICUBIC
+ * One launch covers every job (grid: output tiles x jobs; more than 65535 jobs are launched in slices).  The kernel
+ * computes the coefficients it needs itself; nothing is allocated.  A job whose box or window is empty or outside the
+ * virtual image, or whose virtual size exceeds 2^31 - 1, writes nothing.  Returns BJ_E_ARG for a NULL pointer, n_jobs <= 0, an output size outside 1..65535, an
+ * unknown dtype or an unknown filter.
+ */
+bj_status bj_resize_pil(const bj_resize_pil_job* jobs, int n_jobs, const uint8_t* src, void* dst,
+                        const bj_resize_params* p, int filter, void* stream);
 
 /* ---------------------------------------------------------------------------------------------
  * Reduced-size decode: scale 1/s, s = 2, 4 or 8, in the DCT domain (libjpeg's scale_denom, PIL's draft()).

@@ -463,7 +463,8 @@ extern "C" {
 int bj_version(void) { return BJ_VERSION; }
 int bj_sizeof(int what) {
     return what == 0 ? (int)sizeof(bj_image) : what == 1 ? (int)sizeof(bj_resize_job)
-         : what == 2 ? (int)sizeof(bj_scaled_job) : what == 3 ? (int)sizeof(bj_crop_job) : -1;
+         : what == 2 ? (int)sizeof(bj_scaled_job) : what == 3 ? (int)sizeof(bj_crop_job)
+         : what == 4 ? (int)sizeof(bj_resize_pil_job) : -1;
 }
 const char* bj_last_cuda_error(void) { return g_err; }
 

@@ -2,8 +2,9 @@
 
 The data-loader end of the pipeline: what a training or inference loop feeds a model.  Files are decoded by the
 same batch / streaming pipeline as decode_batch; each decoded sub-batch is resized by one bj_resize launch
-(csrc/bj_resize.cu: antialiased bilinear, like torchvision's Resize) into its slots of the output tensor, after which
-its full-size RGB pixels go back to the allocator.  Memory therefore stays bounded by the sub-batches in flight plus
+(csrc/bj_resize.cu: antialiased bilinear, like torch's antialiased interpolate) or one bj_resize_pil launch
+(csrc/bj_resize_pil.cu: Pillow's Image.resize, bit for bit) into its slots of the output tensor, after which its
+full-size RGB pixels go back to the allocator.  Memory therefore stays bounded by the sub-batches in flight plus
 the output, whatever the number of files.
 """
 from __future__ import annotations
@@ -26,6 +27,21 @@ RESIZE_JOB_DTYPE = np.dtype([
 ])
 assert RESIZE_JOB_DTYPE.itemsize == 40
 
+# numpy mirror of struct bj_resize_pil_job (56 bytes, see include/b200jpeg.h)
+RESIZE_PIL_JOB_DTYPE = np.dtype([
+    ("src_offset", "<u8"), ("src_pitch", "<u4"), ("channels", "<u4"),
+    ("x0", "<u4"), ("y0", "<u4"), ("x1", "<u4"), ("y1", "<u4"),
+    ("dst_index", "<u4"), ("virt_w", "<u4"), ("virt_h", "<u4"), ("win_x", "<u4"), ("win_y", "<u4"),
+    ("reserved", "<u4"),
+])
+assert RESIZE_PIL_JOB_DTYPE.itemsize == 56
+
+# largest virt_w / virt_h of a bj_resize_pil_job
+VIRT_MAX = 2 ** 31 - 1
+
+# resample= of decode_to_tensor -> the filter argument of bj_resize_pil (None: bj_resize)
+RESAMPLES = {"torch": None, "pil-bilinear": 0, "pil-bicubic": 1}
+
 
 class ResizeParams(ctypes.Structure):
     """struct bj_resize_params"""
@@ -44,8 +60,14 @@ def _bind():
         L.bj_resize.restype = ctypes.c_int
         L.bj_resize.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
                                 ctypes.POINTER(ResizeParams), ctypes.c_void_p]
+        L.bj_resize_pil.restype = ctypes.c_int
+        L.bj_resize_pil.argtypes = [ctypes.c_void_p, ctypes.c_int, ctypes.c_void_p, ctypes.c_void_p,
+                                    ctypes.POINTER(ResizeParams), ctypes.c_int, ctypes.c_void_p]
         if L.bj_sizeof(1) != RESIZE_JOB_DTYPE.itemsize:
             raise _native.NativeLibraryError("struct bj_resize_job layout mismatch between Python and libb200jpeg.so")
+        if L.bj_sizeof(4) != RESIZE_PIL_JOB_DTYPE.itemsize:
+            raise _native.NativeLibraryError("struct bj_resize_pil_job layout mismatch between Python and "
+                                             "libb200jpeg.so")
         L._resize_bound = True
     return L
 
@@ -112,6 +134,40 @@ def _fold_norm(dtype, mean, std) -> Tuple[List[float], List[float]]:
     return [1.0 / (255.0 * sv) for sv in s], [-mv / sv for mv, sv in zip(m, s)]
 
 
+def _check_resample(resample, resize, roi, size: Tuple[int, int]) -> Optional[int]:
+    """resample / resize of decode_to_tensor: (resample, resize, roi and size checked) -> the resize= short side or
+    None."""
+    if not isinstance(resample, str) or resample not in RESAMPLES:
+        raise ValueError(f"resample must be one of {', '.join(map(repr, RESAMPLES))}, got {resample!r}")
+    if resize is None:
+        return None
+    if RESAMPLES[resample] is None:
+        raise ValueError("resize= needs resample='pil-bilinear' or 'pil-bicubic'")
+    if roi is not None:
+        raise ValueError("resize= resizes the whole image; it takes roi=None")
+    if isinstance(resize, bool) or not isinstance(resize, (int, np.integer)) or not 1 <= resize <= 65535:
+        raise ValueError(f"resize must be an int in 1..65535, got {resize!r}")
+    if resize < max(size):
+        # the resized short side is `resize`, and either side of an image may be the short one
+        raise ValueError(f"resize={resize} gives images smaller than size={tuple(size)}: it must be >= {max(size)}")
+    return int(resize)
+
+
+def resize_geometry(widths, heights, r: int, size: Tuple[int, int]):
+    """torchvision's Resize(r) then CenterCrop(size) on images of the given sizes: (virt_w, virt_h, win_x, win_y) int64
+    arrays.  The short side becomes r and the long side int(r * long / short) (a square image's width counts as its
+    short side); the crop starts at int(round((virt - out) / 2)) with Python's round (half to even)."""
+    W = np.asarray(widths, dtype=np.int64)
+    H = np.asarray(heights, dtype=np.int64)
+    h, w = size
+    portrait = W <= H
+    short, long = np.where(portrait, W, H), np.where(portrait, H, W)
+    new_long = np.floor(r * long / short).astype(np.int64)    # r * long < 2^53: numpy's division is Python's
+    vw = np.where(portrait, r, new_long)
+    vh = np.where(portrait, new_long, r)
+    return vw, vh, np.round((vw - w) / 2.0).astype(np.int64), np.round((vh - h) / 2.0).astype(np.int64)
+
+
 def pixel_boxes(roi, widths, heights, size: Tuple[int, int]) -> np.ndarray:
     """(n, 4) int64 pixel boxes (px0, py0, px1, py1) of images of the given sizes for a checked roi (_check_roi)."""
     W = np.asarray(widths, dtype=np.int64)
@@ -153,11 +209,13 @@ def _resize_stream(dev: torch.device) -> torch.cuda.Stream:
 
 
 class _Resizer:
-    """Enqueues bj_resize for decoded sub-batches into the slots of one output tensor, on the resize stream."""
+    """Enqueues bj_resize (filter None) or bj_resize_pil for decoded sub-batches into the slots of one output tensor, on
+    the resize stream.  resize: the resize= short side (bj_resize_pil only) or None."""
 
-    def __init__(self, out: torch.Tensor, roi, size, dtype, a, b, channels_last: bool):
+    def __init__(self, out: torch.Tensor, roi, size, dtype, a, b, channels_last: bool, filter_=None, resize=None):
         self.L = _bind()
         self.out, self.roi, self.size = out, roi, size
+        self.filter, self.resize_to = filter_, resize
         self.dev = out.device
         self.stream = _resize_stream(self.dev)
         self.params = ResizeParams(size[0], size[1], DTYPES[dtype], int(channels_last), (ctypes.c_float * 3)(*a),
@@ -177,12 +235,25 @@ class _Resizer:
         if isinstance(roi, np.ndarray) and roi.ndim == 2:
             roi = roi[np.fromiter((s for _, s in items), dtype=np.int64, count=len(items))]
         boxes = pixel_boxes(roi, W, H, self.size)
-        jobs = np.zeros(len(items), dtype=RESIZE_JOB_DTYPE)
+        jobs = np.zeros(len(items), dtype=RESIZE_JOB_DTYPE if self.filter is None else RESIZE_PIL_JOB_DTYPE)
         jobs["src_offset"] = lay.offsets[idx]
         jobs["src_pitch"] = lay.pitches[idx]
         jobs["channels"] = lay.channels[idx]
         jobs["x0"], jobs["y0"], jobs["x1"], jobs["y1"] = boxes[:, 0], boxes[:, 1], boxes[:, 2], boxes[:, 3]
         jobs["dst_index"] = [s for _, s in items]
+        if self.filter is not None:
+            if self.resize_to is None:
+                jobs["virt_w"], jobs["virt_h"] = self.size[1], self.size[0]
+            else:
+                vw, vh, wx, wy = resize_geometry(boxes[:, 2] - boxes[:, 0], boxes[:, 3] - boxes[:, 1], self.resize_to,
+                                                 self.size)
+                too_long = np.flatnonzero(np.maximum(vw, vh) > VIRT_MAX)
+                if too_long.size:        # checked before the launch: the kernel writes nothing for such a job
+                    k = int(too_long[0])
+                    raise ValueError(f"resize={self.resize_to} makes the {int(boxes[k, 2] - boxes[k, 0])} x "
+                                     f"{int(boxes[k, 3] - boxes[k, 1])} image {int(max(vw[k], vh[k]))} pixels long, "
+                                     f"more than {VIRT_MAX}")
+                jobs["virt_w"], jobs["virt_h"], jobs["win_x"], jobs["win_y"] = vw, vh, wx, wy
         staged = torch.empty(jobs.nbytes, dtype=torch.uint8, pin_memory=True)
         staged.numpy()[:] = jobs.view(np.uint8)
         s = self.stream
@@ -191,8 +262,14 @@ class _Resizer:
                 s.wait_stream(after)
             dev_jobs = torch.empty(jobs.nbytes, dtype=torch.uint8, device=self.dev)
             dev_jobs.copy_(staged, non_blocking=True)    # the pinned block is kept until this copy has completed
-            _native.check(self.L.bj_resize(dev_jobs.data_ptr(), len(items), batch.out.data_ptr(), self.out.data_ptr(),
-                                           ctypes.byref(self.params), s.cuda_stream), "bj_resize")
+            if self.filter is None:
+                _native.check(self.L.bj_resize(dev_jobs.data_ptr(), len(items), batch.out.data_ptr(),
+                                               self.out.data_ptr(), ctypes.byref(self.params), s.cuda_stream),
+                              "bj_resize")
+            else:
+                _native.check(self.L.bj_resize_pil(dev_jobs.data_ptr(), len(items), batch.out.data_ptr(),
+                                                   self.out.data_ptr(), ctypes.byref(self.params), self.filter,
+                                                   s.cuda_stream), "bj_resize_pil")
             batch.out.record_stream(s)                   # the RGB buffer may be reused only after the resize has read it
 
     def finish(self) -> None:
@@ -201,7 +278,7 @@ class _Resizer:
 
 def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtype=torch.float32, mean=None, std=None,
                      channels_last: bool = False, device=None, chunk: Optional[int] = None, on_error: str = "raise",
-                     scale=1, compat: str = "reference"):
+                     scale=1, compat: str = "reference", resample: str = "torch", resize: Optional[int] = None):
     """Decode `files` (paths or bytes, like decode_batch) into ONE device tensor of shape (N, 3, h, w), (h, w) = size.
 
     Each image's region `roi` is resized like torch.nn.functional.interpolate(mode="bilinear", antialias=True,
@@ -221,6 +298,14 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
                 still at least (h, w), so nothing is upscaled that the full decode would have downscaled.
       compat    "reference", or "libjpeg-turbo": the resize reads libjpeg-turbo's pixels (Pillow's), scale 1 only
                 (decode_batch(compat=)).
+      resample  "torch" (the resize above), or "pil-bilinear" / "pil-bicubic": each image's box is resized exactly like
+                PIL.Image.resize((w, h), BILINEAR | BICUBIC) of the decoded box (torchvision's resized_crop on a PIL
+                image).  uint8 output holds Pillow's bytes; float outputs are v * a[c] + b[c] of those uint8 values v,
+                so with compat="libjpeg-turbo" they equal ToTensor() + Normalize() up to fp32 rounding.
+      resize    an int r, PIL resamples only, roi=None, r >= max(h, w): torchvision's Resize(r) then CenterCrop(size)
+                -- the short side becomes r, the long side int(r * long / short), the crop starts at
+                int(round((R - h) / 2)), int(round((C - w) / 2)) -- of which only the cropped window is computed.
+                With scale="auto" each file uses the largest scale whose decoded short side is still >= r.
     With a roi, only each file's roi box is decoded (decode_batch(crop=)), taken at the scale the file uses; the
     resize then reads the whole decoded crop, which holds the same bytes as the box of the full decode.
     The caller's current stream is ordered after the work, so the tensor can be used right away."""
@@ -236,12 +321,13 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
     files = list(files)
     n = len(files)
     roi = _check_roi(roi, n)
+    resize = _check_resample(resample, resize, roi, (h, w))
     chunk = BATCH_CHUNK if chunk is None else int(chunk)
     if chunk < 1:
         raise ValueError("chunk must be positive")
     scales = None if scale == 1 else scale
     if scale == "auto":
-        scales = _AutoScales(roi, (h, w))
+        scales = _AutoScales(roi, (h, w) if resize is None else (resize, resize))
     crops = None if roi is None else _RoiCrops(roi, (h, w), scales)
 
     from .stages import require_cuda
@@ -255,7 +341,8 @@ def decode_to_tensor(files: Sequence[Source], size=(224, 224), *, roi=None, dtyp
             out.zero_()
         if n == 0:
             return (out, []) if on_error == "return" else out
-        rs = _Resizer(out, None if crops is not None else roi, (h, w), dtype, a, b, channels_last)
+        rs = _Resizer(out, None if crops is not None else roi, (h, w), dtype, a, b, channels_last, RESAMPLES[resample],
+                      resize)
         cur = torch.cuda.current_stream(dev)
         # finish() also runs when a file raises part-way: resizes already enqueued may still be writing into `out`,
         # which the caller's stream must not reuse before they are done
